@@ -17,6 +17,11 @@ every rank its own batch of M points instead (reported as a secondary block in t
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--scaling strong|weak]
                   [--nh 1024 --nl 4096 --points 1048576 --samples 100] [--no-lml] [--no-cpu] [--no-extras]
+                  [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed step returned -- the per-point predictive mean and variance
+and the PCE mean -- as float64 DIR/<name>.npy (DIR/<name>_rank<r>.npy under torchrun), so that two builds run
+with the same arguments (same seeded inputs) can be compared output for output.
 """
 import os
 import sys
@@ -643,6 +648,27 @@ def per_row_reference_loop(wl, n_rows):
             "max_abs_diff_vs_vectorised": float(np.max(np.abs(mean - mean_v)))}
 
 
+DUMP_MAX_BYTES = 64 * 10 ** 6         # all files of one --dump-outputs together
+
+
+def write_outputs(path, per_point, other, max_bytes=DUMP_MAX_BYTES, suffix=""):
+    """Write every array as float64 path/<name><suffix>.npy.  per_point: arrays whose first axis runs over
+    the test points; when the files would exceed max_bytes they are cut to the same fixed, seeded sample
+    of rows (ascending), whose row indices go to index<suffix>.npy (as float64, exact below 2^53)."""
+    os.makedirs(path, exist_ok=True)
+    per_point = {k: np.asarray(v, dtype=np.float64) for k, v in per_point.items()}
+    other = {k: np.asarray(v, dtype=np.float64) for k, v in other.items()}
+    budget = max_bytes - 128 * (len(per_point) + len(other) + 1) - sum(v.nbytes for v in other.values())
+    if sum(v.nbytes for v in per_point.values()) > budget:              # 128: one .npy header per file
+        n = len(next(iter(per_point.values())))
+        row_bytes = 8 + sum(v.nbytes // n for v in per_point.values())      # + 8: the row's index
+        keep = np.sort(np.random.default_rng(0).choice(n, budget // row_bytes, replace=False))
+        per_point = {k: v[keep] for k, v in per_point.items()}
+        other["index"] = keep.astype(np.float64)
+    for k, v in {**per_point, **other}.items():
+        np.save(os.path.join(path, k + suffix + ".npy"), v)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -660,7 +686,11 @@ def main():
     ap.add_argument("--no-lml", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="headline only (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
 
     if args.impl == "reference":
         run_reference(args)
@@ -744,7 +774,7 @@ def main():
 
         def step_device():
             mean, var, wsum = model.predict_mc_device(dX, S, None, 2, m0, dw)
-            return reduce_pce(wsum)
+            return reduce_pce(wsum), mean, var
 
         def step_e2e():
             # public API, host buffers: pinned NumPy views in, NumPy out (H2D + D2H inside the timed region)
@@ -752,7 +782,7 @@ def main():
             return reduce_pce(model.last_pce_mean), mean, var
 
         for _ in range(warmup):
-            pce = step_device()
+            step_device()
         sampler = ClockSampler(local) if (rank == 0 and sample_clocks) else None
         barrier()
         if sampler:
@@ -762,7 +792,7 @@ def main():
         s_ev, e_ev = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         s_ev.record()
         for _ in range(steps):
-            pce = step_device()
+            pce, mean, var = step_device()
         e_ev.record()
         barrier()
         launches = h.launches - launches0
@@ -772,7 +802,8 @@ def main():
         clocks = sampler.stop() if sampler else None
         total = float(M) * S * (1 if strong_mode else world)
         res = {"ms_dev": ms_dev, "value": total / (ms_dev * 1e-3), "pce": pce, "launches": launches, "prof": prof,
-               "clocks": clocks, "points_per_rank": hi - lo, "total_samples": total}
+               "clocks": clocks, "points_per_rank": hi - lo, "total_samples": total,
+               "outputs": {"mean": mean.cpu().numpy(), "var": var.cpu().numpy()}}
         if with_e2e:
             step_e2e()
             barrier()
@@ -790,6 +821,9 @@ def main():
         return res
 
     main_res = run_mode(strong, args.steps, args.warmup, True, True)
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, main_res["outputs"], {"pce_mean": np.array([main_res["pce"]])},
+                      max_bytes=DUMP_MAX_BYTES // world, suffix="_rank%d" % rank if world > 1 else "")
     weak_res = None
     if world > 1 and strong and not args.no_extras:
         weak_res = run_mode(False, 2, 1, False, False)       # secondary: every rank its own M points
