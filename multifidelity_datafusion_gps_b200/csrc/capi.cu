@@ -1,6 +1,5 @@
 // extern "C" entry points declared in include/mfgp_b200.h: argument checks, scratch layout,
 // chunk loops and stream ordering.  No torch types, no allocation outside mfgp_create.
-#include <stdlib.h>
 #include <time.h>
 #include "common.cuh"
 
@@ -150,15 +149,6 @@ int make_kparams(mfgp_ctx* h, int kind, int D, int d, const double* theta, int P
 // Up to this size the single-CTA kernel beats the multi-kernel chain (wall time per LML+gradient evaluation:
 // N = 8: 66 vs 92 us, N = 30: 78 vs 108 us, N = 100: 147 vs 144 us; tools/fit_time.py)
 #define MFGP_SMALL_N 96
-// MFGP_SMALL_PATH=0 routes these sizes through the multi-kernel chain as well (A/B and parity checks)
-static bool small_path() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("MFGP_SMALL_PATH");
-    v = (e && atoi(e) == 0) ? 0 : 1;
-  }
-  return v == 1;
-}
 
 static int fetch_scalars(mfgp_ctx* h, int ndoubles) {
   CUDA_TRY(h, cudaMemcpyAsync(h->h_pinned, h->d_scalars, ndoubles * sizeof(double),
@@ -351,7 +341,7 @@ int mfgp_factorize(mfgp_handle_t h, int kind, const double* d_X, const double* d
   KParams kp;
   int rc = make_kparams(h, kind, D, d, h_theta, P, &kp);
   if (rc) return rc;
-  if (N <= MFGP_SMALL_N && small_path()) {
+  if (N <= MFGP_SMALL_N) {
     if ((rc = small_gp_launch(h, kp, d_X, d_y, N, kp.noise + JITTER_CONST + jitter, d_A, d_W, d_alpha,
                               h->d_scalars, 0)))
       return rc;
@@ -393,7 +383,7 @@ int mfgp_lml_grad_timed(mfgp_handle_t h, int kind, const double* d_X, const doub
   int rc = make_kparams(h, kind, D, d, h_theta, P, &kp);
   if (rc) return rc;
   const int npad = mfgp_padded_n(N);
-  if (N <= MFGP_SMALL_N && small_path()) {   // one fused launch; no per-stage times
+  if (N <= MFGP_SMALL_N) {   // one fused launch; no per-stage times
     if ((rc = small_gp_launch(h, kp, d_X, d_y, N, kp.noise + JITTER_CONST + jitter, d_A, d_W, d_alpha,
                               h->d_scalars, 1)))
       return rc;
@@ -408,8 +398,7 @@ int mfgp_lml_grad_timed(mfgp_handle_t h, int kind, const double* d_X, const doub
   // Untimed (production) schedule: the O(N^2), HBM-bound solves (v = W y, alpha = W^T v, LML) run on the side stream
   // UNDER the tensor-bound K^-1 = W^T W -- both only read W.  With stage timing the schedule stays sequential so
   // that the six stage times add up.
-  static const bool overlap_solve = !(getenv("MFGP_OVERLAP_SOLVE") && atoi(getenv("MFGP_OVERLAP_SOLVE")) == 0);
-  if (!ev && overlap_solve && h->s_hi && npad >= 2048 && 2LL * npad <= MFGP_PARTIALS) {
+  if (!ev && h->s_hi && npad >= 2048 && 2LL * npad <= MFGP_PARTIALS) {
     if ((rc = factor_enqueue(h, kp, d_X, d_y, N, jitter, d_A, d_W, d_alpha, nullptr, true))) return rc;
     cudaStream_t caller = h->stream;
     cudaEvent_t ev_fork = h->ev_la[3 * 64], ev_join = h->ev_la[3 * 64 + 1];
@@ -794,14 +783,11 @@ static int mc_chain_impl(mfgp_ctx* h, const mfgp_level_t* const* levels, int L, 
   // the trmm_sumsq / cross_gen classes hold the high-fidelity launches only)
   const int prof_saved = h->prof_on;
   h->prof_on = 0;
-  static const bool trace = getenv("MFGP_TRACE_MC") != nullptr;   // stage times to stderr (diagnostics)
-  if (trace) cudaEventRecord(h->ev[0], h->stream);
   rc = predict_impl(h, lf, kp[0], d_Xtest, M, mu_l, sd_l, include_lower_noise, rest,
                     (size_t)restd * sizeof(double));
   h->prof_on = prof_saved;
   if (rc) return rc;
   if ((rc = sqrt_launch(h, sd_l, M))) return rc;
-  if (trace) cudaEventRecord(h->ev[1], h->stream);
   // upper levels over (point, sample) columns
   const int D = d + 1;
   // when every upper level takes the fused small-level kernel no cross-covariance row is ever stored: a column
@@ -862,15 +848,6 @@ static int mc_chain_impl(mfgp_ctx* h, const mfgp_level_t* const* levels, int L, 
       if ((rc = finish_var_launch(h, ss, ncols, kp[t].kdiag, with_noise ? kp[t].noise : 0.0, ss))) return rc;
     }
     if ((rc = mc_aggregate_launch(h, mu_c, ss, npts, S, d_mean + m_lo, d_var + m_lo))) return rc;
-  }
-  if (trace) {
-    cudaEventRecord(h->ev[2], h->stream);
-    cudaEventSynchronize(h->ev[2]);
-    float lf_ms = 0.f, hf_ms = 0.f;
-    cudaEventElapsedTime(&lf_ms, h->ev[0], h->ev[1]);
-    cudaEventElapsedTime(&hf_ms, h->ev[1], h->ev[2]);
-    fprintf(stderr, "[mfgp trace] predict_mc M=%lld S=%d: lowest level %.2f ms, upper levels %.2f ms\n", M, S, lf_ms,
-            hf_ms);
   }
   if (h_wsum) {
     if ((rc = wdot_launch(h, d_weights, d_mean, M, h->d_scalars + 20))) return rc;

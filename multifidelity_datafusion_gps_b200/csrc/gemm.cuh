@@ -5,7 +5,7 @@
 // DMMA.8x8x4 fed from shared memory.  The core is a BMxBNx32 CTA tile with a 3-stage cp.async
 // (LDGSTS) pipeline (measured against 16-deep / 4 stages: fewer barriers per flop, deeper prefetch:
 // +1.5 % on every GEMM) and conflict-free padded shared-memory layouts; instantiations:
-//   Big   128x128, 8 warps of 64x32  -- throughput shape (1 CTA / SM, 216 KB smem)
+//   Big16 128x128, 16 warps of 32x32 -- throughput shape (1 CTA / SM, 216 KB smem)
 //   Small  64x64,  4 warps of 32x32  -- latency shape for the narrow GEMMs on the critical path of the
 //                                       recursive factorisation (4x the CTAs, 2 CTAs / SM)
 //
@@ -44,8 +44,7 @@ struct TileCfg {
   static constexpr int STAGE_DOUBLES = A_STAGE + B_STAGE;
   static constexpr int SMEM_BYTES = STAGES * STAGE_DOUBLES * 8;
 };
-using Big = TileCfg<128, 128, 2, 4>;     // 221184 B smem
-using Big16 = TileCfg<128, 128, 4, 4>;   // same tile, 16 warps of 32x32 (4 warps per scheduler)
+using Big16 = TileCfg<128, 128, 4, 4>;   // 221184 B smem, 16 warps of 32x32 (4 warps per scheduler)
 using Small = TileCfg<64, 64, 2, 2>;     // 110592 B smem
 using Row32 = TileCfg<32, 128, 1, 4>;    // 138240 B smem: owns all 128 columns of its 32 rows (in-place TRSM leaf)
 

@@ -9,22 +9,8 @@
 //              inverse); A22 -= A21 A21^T (SYRK, lower tiles); potrf(A22)
 //   trtri(n):  trtri(11), trtri(22); W21 = -W22 L21 W11
 //   lauum:     Kinv = W^T W, one launch over the lower tiles with k >= row0
-#include <stdlib.h>
 #include "gemm.cuh"
 #include "fastmath.cuh"
-
-#ifndef MFGP_TRMM_TMA_DEFAULT
-#define MFGP_TRMM_TMA_DEFAULT 1      // measured r02: 2.42 -> 2.27 ms per 75 776 x 1024 launch, bit-identical sums
-#endif
-#ifndef MFGP_NARROW_BIG_M_DEFAULT
-#define MFGP_NARROW_BIG_M_DEFAULT 6144      // measured r02 at N = 16384: potrf 50.3 -> 48.7 ms (8192: 49.0, 4096: 48.9, 2048: 49.5, 0: 50.0)
-#endif
-#ifndef MFGP_GEMM_TMA_MC_DEFAULT
-#define MFGP_GEMM_TMA_MC_DEFAULT 1
-#endif
-#ifndef MFGP_GEMM_TMA_DEFAULT
-#define MFGP_GEMM_TMA_DEFAULT 1      // measured r02 at N = 16384: potrf 53.8 -> 51.6 ms, trtri 44.7 -> 43.6, same bits
-#endif
 
 namespace {
 
@@ -586,16 +572,6 @@ __global__ void __launch_bounds__(256, 1)
   }
 }
 
-// A/B switch for the throughput tile (environment MFGP_TILE_WARPS=8|16), read once
-int tile_variant() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("MFGP_TILE_WARPS");
-    v = (e && atoi(e) == 8) ? 8 : 16;
-  }
-  return v;
-}
-
 template <class T>
 int tile_count(const dg::GemmParams& p) {
   const int tm = p.M / T::BM, tn = p.N / T::BN;
@@ -634,38 +610,10 @@ static bool make_map(CUtensorMap* m, const double* base, unsigned long long inne
             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-// MFGP_TRMM_TMA=1|0 selects the TMA + mbarrier variant of trmm_sumsq, MFGP_GEMM_TMA=1|0 that of the NT GEMMs
-// (read once)
-static int trmm_tma_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("MFGP_TRMM_TMA");
-    v = e ? (atoi(e) != 0) : MFGP_TRMM_TMA_DEFAULT;
-  }
-  return v;
-}
-static int gemm_neg_init() {     // MFGP_GEMM_NEG_INIT=0: read-modify-write epilogue for C -= A B^T
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("MFGP_GEMM_NEG_INIT");
-    v = e ? (atoi(e) != 0) : 1;
-  }
-  return v;
-}
-static int gemm_tma_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("MFGP_GEMM_TMA");
-    v = e ? (atoi(e) != 0) : MFGP_GEMM_TMA_DEFAULT;
-  }
-  return v;
-}
-
-
 // NT product through the TMA kernel (k-contiguous operands, full 128 x 128 tiles on at least one wave).
-// Returns 1 if it took the launch.
+// Returns 1 if it took the launch.  Measured r02 against the cp.async kernels at N = 16384: potrf 53.8 -> 51.6 ms,
+// trtri 44.7 -> 43.6, same bits.
 static int try_gemm_tma(mfgp_ctx* h, const dg::GemmParams& p, int cls) {
-  if (!gemm_tma_enabled()) return 0;
   const int nodes = p.batch > 1 ? p.batch : 1;
   // operand views: A is (M + node shifts) x K, B is (N + node shifts) x K; the leading dimension bounds k
   const long shift = nodes > 1 ? p.batch_stride : 0;      // elements per node along the diagonal: n * (ld + 1)
@@ -690,7 +638,7 @@ static int try_gemm_tma(mfgp_ctx* h, const dg::GemmParams& p, int cls) {
   q.batch = p.batch; q.c_batch_stride = c_stride;
   q.a_batch_rows = (int)a_rows_shift; q.a_batch_k = (int)a_k_shift;
   q.b_batch_rows = (int)b_rows_shift; q.b_batch_k = (int)b_k_shift;
-  q.neg_init = gemm_neg_init() && p.alpha == -1.0 && p.beta == 1.0;
+  q.neg_init = p.alpha == -1.0 && p.beta == 1.0;
   prof_begin(h, cls);
   dg::gemm_tma_kernel<dg::Big16><<<tile_count<dg::Big16>(p), dg::Big16::THREADS, dg::tma::SMEM_BYTES, h->stream>>>(
       tmA, tmB, q);
@@ -712,21 +660,11 @@ static bool make_map_mc(CUtensorMap* m, const double* base, unsigned long long m
             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-static int gemm_tma_mc_enabled() {     // MFGP_GEMM_TMA_MC=0: cp.async kernels for the TN / TT / NN products
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("MFGP_GEMM_TMA_MC");
-    v = e ? (atoi(e) != 0) : MFGP_GEMM_TMA_MC_DEFAULT;
-  }
-  return v;
-}
-
 // Products with at least one m-contiguous operand (first product of the triangular inverse, K^-1 = W^T W,
 // the Gram / right-multiply helpers of the delayed-input MC path) through gemm_tma_mc_kernel.  Returns 1 if it
 // took the launch.
 template <bool A_KC, bool B_KC>
 static int try_gemm_tma_mc(mfgp_ctx* h, const dg::GemmParams& p, int cls) {
-  if (!gemm_tma_enabled() || !gemm_tma_mc_enabled()) return 0;
   const int nodes = p.batch > 1 ? p.batch : 1;
   long n_shift = 0, c_stride = 0;
   if (nodes > 1) {
@@ -760,28 +698,21 @@ static int try_gemm_tma_mc(mfgp_ctx* h, const dg::GemmParams& p, int cls) {
 // Narrow products of the Cholesky panel (row solves, in-panel updates: fewer 128 x 128 tiles than SMs).  With many
 // rows below the panel the bulk update hides the panel, and what these products cost is MACHINE time: full 128 x 128
 // TMA tiles (one CTA per 128 rows) do the same flops on a quarter of the SM time of the 64 x 64 / 32 x 128 latency
-// tiles, which are kept for the chain-bound tail.  MFGP_NARROW_BIG_M = rows from which the big tiles are used.
-static int narrow_big_rows() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("MFGP_NARROW_BIG_M");
-    v = e ? atoi(e) : MFGP_NARROW_BIG_M_DEFAULT;
-    if (v < 0) v = 1 << 30;
-  }
-  return v;
-}
+// tiles, which are kept for the chain-bound tail.  NARROW_BIG_ROWS = rows from which the big tiles are used; measured
+// r02 at N = 16384: potrf 50.3 -> 48.7 ms (8192: 49.0, 4096: 48.9, 2048: 49.5, 0: 50.0).
+constexpr int NARROW_BIG_ROWS = 6144;
 
 template <bool A_KC, bool B_KC>
 int launch_gemm(mfgp_ctx* h, const dg::GemmParams& p, int cls = PC_GEMM) {
-  const int big_tiles = tile_count<dg::Big>(p);
+  const int big_tiles = tile_count<dg::Big16>(p);
   if (big_tiles <= 0) return 0;
-  if (A_KC && B_KC && tile_variant() == 16 &&
-      (big_tiles >= MFGP_NUM_SMS || (p.batch <= 1 && p.M >= narrow_big_rows())) && try_gemm_tma(h, p, cls)) {
+  if (A_KC && B_KC && (big_tiles >= MFGP_NUM_SMS || (p.batch <= 1 && p.M >= NARROW_BIG_ROWS)) &&
+      try_gemm_tma(h, p, cls)) {
     LAUNCH_CHECK(h);
     return 0;
   }
   if constexpr (!(A_KC && B_KC)) {
-    if (big_tiles >= MFGP_NUM_SMS && tile_variant() == 16 && try_gemm_tma_mc<A_KC, B_KC>(h, p, cls)) {
+    if (big_tiles >= MFGP_NUM_SMS && try_gemm_tma_mc<A_KC, B_KC>(h, p, cls)) {
       LAUNCH_CHECK(h);
       return 0;
     }
@@ -790,12 +721,9 @@ int launch_gemm(mfgp_ctx* h, const dg::GemmParams& p, int cls = PC_GEMM) {
   if (big_tiles < MFGP_NUM_SMS) {
     dg::gemm_kernel<dg::Small, A_KC, B_KC>
         <<<tile_count<dg::Small>(p), dg::Small::THREADS, dg::Small::SMEM_BYTES, h->stream>>>(p);
-  } else if (tile_variant() == 16) {
+  } else {
     dg::gemm_kernel<dg::Big16, A_KC, B_KC>
         <<<big_tiles, dg::Big16::THREADS, dg::Big16::SMEM_BYTES, h->stream>>>(p);
-  } else {
-    dg::gemm_kernel<dg::Big, A_KC, B_KC>
-        <<<big_tiles, dg::Big::THREADS, dg::Big::SMEM_BYTES, h->stream>>>(p);
   }
   prof_end(h, cls);
   LAUNCH_CHECK(h);
@@ -805,7 +733,7 @@ int launch_gemm(mfgp_ctx* h, const dg::GemmParams& p, int cls = PC_GEMM) {
 // X <- X * Wl^T in place (X: m x 128, Wl: 128 x 128): every CTA must own all 128 columns of its rows
 int launch_trsm_leaf(mfgp_ctx* h, const dg::GemmParams& p) {
   // (in place is safe with the TMA kernel too: a CTA owns all 128 columns of its rows and stores after its last slab)
-  if (tile_variant() == 16 && p.M >= narrow_big_rows() && try_gemm_tma(h, p, PC_GEMM)) {
+  if (p.M >= NARROW_BIG_ROWS && try_gemm_tma(h, p, PC_GEMM)) {
     LAUNCH_CHECK(h);
     return 0;
   }
@@ -814,8 +742,8 @@ int launch_trsm_leaf(mfgp_ctx* h, const dg::GemmParams& p) {
     dg::gemm_kernel<dg::Row32, true, true>
         <<<tile_count<dg::Row32>(p), dg::Row32::THREADS, dg::Row32::SMEM_BYTES, h->stream>>>(p);
   } else {
-    dg::gemm_kernel<dg::Big, true, true>
-        <<<tile_count<dg::Big>(p), dg::Big::THREADS, dg::Big::SMEM_BYTES, h->stream>>>(p);
+    dg::gemm_kernel<dg::Big16, true, true>
+        <<<tile_count<dg::Big16>(p), dg::Big16::THREADS, dg::Big16::SMEM_BYTES, h->stream>>>(p);
   }
   prof_end(h, PC_GEMM);
   LAUNCH_CHECK(h);
@@ -912,10 +840,6 @@ static int configure_gemm(mfgp_ctx* h) {
 
 int linalg_configure(mfgp_ctx* h) {
   int rc = 0;
-  rc |= configure_gemm<dg::Big, true, true>(h);
-  rc |= configure_gemm<dg::Big, false, true>(h);
-  rc |= configure_gemm<dg::Big, false, false>(h);
-  rc |= configure_gemm<dg::Big, true, false>(h);
   rc |= configure_gemm<dg::Small, true, false>(h);
   rc |= configure_gemm<dg::Big16, true, false>(h);
   rc |= configure_gemm<dg::Small, true, true>(h);
@@ -923,8 +847,6 @@ int linalg_configure(mfgp_ctx* h) {
   rc |= configure_gemm<dg::Small, false, false>(h);
   rc |= configure_gemm<dg::Row32, true, true>(h);
   if (rc) return -100;
-  CUDA_TRY(h, cudaFuncSetAttribute(dg::trmm_sumsq_kernel<dg::Big>,
-                                   cudaFuncAttributeMaxDynamicSharedMemorySize, dg::Big::SMEM_BYTES));
   CUDA_TRY(h, cudaFuncSetAttribute(dg::trmm_sumsq_kernel<dg::Big16>,
                                    cudaFuncAttributeMaxDynamicSharedMemorySize, dg::Big16::SMEM_BYTES));
   CUDA_TRY(h, cudaFuncSetAttribute(dg::trmm_sumsq_tma_kernel<dg::Big16>,
@@ -952,26 +874,22 @@ int linalg_configure(mfgp_ctx* h) {
 // trailing update runs on the caller's stream and overlaps the critical path of panel p+1.
 //   la[p]   (s_hi)  : A[next block column] -= L21 L21[next rows]^T      waits bulk[p-1] (same tiles)
 //   bulk[p] (s_main): A[beyond next block column, lower] -= L21 L21^T   waits trsm[p]
-static int LA_NB_ENV = 0;     // MFGP_LA_NB overrides the panel width (multiple of 128) for tuning
 constexpr int LA_MIN = 4096;    // below this the plain recursion is as fast
 constexpr int LA_MAXP = 64;
-// measured at N = 16384: 512 -> 55.1 ms, 768 -> 55.4, 1024 -> 56.3, 2048 -> 61.2 (profiles/r01_notes.md)
-// MFGP_LA_TAIL: remaining columns at which the plain recursion would take over from the panels.  Measured at
-// N = 16384 (profiles/r02_potrf_tail.txt): 0 -> 53.8 ms, 2048 -> 53.9, 4096 -> 54.6, 6144 -> 56.0, 8192 -> 57.8:
-// the recursion loses at every size (its half-size TRSM / SYRK expose MORE serial leaf chain, not less), so the
-// switch stays off; kept for the record and for other shapes.
-static int LA_TAIL = 0;
+// Panel width, measured at N = 16384: 512 -> 55.1 ms, 768 -> 55.4, 1024 -> 56.3, 2048 -> 61.2 (profiles/r01_notes.md)
 // (r02, with the big-tile policy for hidden panels: N = 16384: 512 -> 49.0 ms, 640 -> 49.0, 768 -> 49.4, 1024 -> 50.0;
 //  N = 32768: 512 -> 353.6 ms, 1024 -> 344.8)
-static int la_nb(int npad) { return LA_NB_ENV ? LA_NB_ENV : (npad < 24576 ? 512 : 1024); }
+static int la_nb(int npad) { return npad < 24576 ? 512 : 1024; }
+// The panels run to the last column.  Handing the remaining columns to the plain recursion was measured at
+// N = 16384 (profiles/r02_potrf_tail.txt), by the number of remaining columns: never -> 53.8 ms, 2048 -> 53.9,
+// 4096 -> 54.6, 6144 -> 56.0, 8192 -> 57.8: the recursion loses at every size (its half-size TRSM / SYRK expose
+// MORE serial leaf chain, not less).
 
 // The panel's critical path, 128 columns at a time (left-looking inside the panel): leaf -> ONE in-place
 // multiply of ALL rows below by the leaf inverse -> ONE update of the next 128-column block by the panel
 // columns factorised so far.  12 launches per 512-column panel against 20 for potrf_rec + trsm_rec (whose
 // recursion buys nothing here: every one of its GEMMs is narrower than the machine, so each costs a launch
 // latency whatever its size), i.e. a shorter serial chain wherever the bulk update no longer hides it.
-// MFGP_LA_CHAIN=0 restores the recursive panel.
-static int LA_CHAIN = 1;
 static int panel_chain(mfgp_ctx* h, double* A, double* W, long ld, int c0, int w, int npad, int nreal) {
   int rc = 0;
   for (int j = 0; j < w && rc == 0; j += LEAF) {
@@ -1010,28 +928,10 @@ static int potrf_lookahead(mfgp_ctx* h, double* A, double* W, int npad, int nrea
   const int P = (npad + LA_NB - 1) / LA_NB;
   for (int p = 0; p < P && rc == 0; p++) {
     const int c0 = p * LA_NB;
-    if (p > 0 && npad - c0 <= LA_TAIL) {
-      // Tail: the trailing block is so small that a bulk update (a few hundred tiles) is shorter than the
-      // serial panel chain it should hide, so every further panel would cost its whole ~0.7 ms chain.  The
-      // plain recursion factorises such a block faster (its TRSM / SYRK are wide, and half of the leaves
-      // sit in the first half, ahead of any update): finish the remaining block with it, after both streams
-      // have delivered panel p-1's updates.
-      CUDA_TRY(h, cudaEventRecord(ev_trsm[p], s_hi));
-      CUDA_TRY(h, cudaStreamWaitEvent(s_main, ev_trsm[p], 0));
-      h->stream = s_main;
-      rc = potrf_rec(h, A, W, ld, c0, npad - c0, nreal);
-      break;
-    }
     const int w = (npad - c0 < LA_NB) ? npad - c0 : LA_NB;
     const int m = npad - c0 - w;
     h->stream = s_hi;
-    if (LA_CHAIN) {
-      rc = panel_chain(h, A, W, ld, c0, w, npad, nreal);
-    } else {
-      rc = potrf_rec(h, A, W, ld, c0, w, nreal);
-      if (rc == 0 && m > 0) rc = trsm_rec(h, A, W, ld, c0 + w, m, c0, w);
-    }
-    if (rc) break;
+    if ((rc = panel_chain(h, A, W, ld, c0, w, npad, nreal))) break;
     if (m > 0) {
       CUDA_TRY(h, cudaEventRecord(ev_trsm[p], s_hi));
       const int w2 = m < LA_NB ? m : LA_NB;
@@ -1066,24 +966,10 @@ static int potrf_lookahead(mfgp_ctx* h, double* A, double* W, int npad, int nrea
   return rc;
 }
 
-static int USE_LA = -1;
-static void potrf_env() {     // tuning switches, read once
-  if (USE_LA >= 0) return;
-  const char* e = getenv("MFGP_LOOKAHEAD");
-  USE_LA = (e && atoi(e) == 0) ? 0 : 1;
-  const char* tl = getenv("MFGP_LA_TAIL");
-  if (tl && atoi(tl) >= 0) LA_TAIL = atoi(tl);
-  const char* ch = getenv("MFGP_LA_CHAIN");
-  if (ch) LA_CHAIN = atoi(ch) != 0;
-  const char* nb = getenv("MFGP_LA_NB");
-  if (nb && atoi(nb) >= 128 && atoi(nb) % 128 == 0) LA_NB_ENV = atoi(nb);
-}
-
 int potrf_padded(mfgp_ctx* h, double* A, double* W, int npad, int nreal) {
   ARG_CHECK(h, npad > 0 && npad % LEAF == 0);
   CUDA_TRY(h, cudaMemsetAsync(h->d_info, 0, 4 * sizeof(int), h->stream));
-  potrf_env();
-  if (USE_LA && h->s_hi && npad >= LA_MIN && npad <= la_nb(npad) * LA_MAXP) {
+  if (h->s_hi && npad >= LA_MIN && npad <= la_nb(npad) * LA_MAXP) {
     cudaStream_t caller = h->stream;
     const int rc = potrf_lookahead(h, A, W, npad, nreal);
     h->stream = caller;   // also on the error paths inside
@@ -1146,20 +1032,13 @@ int trtri_padded(mfgp_ctx* h, const double* L, double* W, int npad) {
 // updates move to a medium-priority stream and the chain keeps the high-priority one.  Same products on the same
 // data as potrf_padded + trtri_padded; a level batched over half of the matrix may fall below one wave of tiles
 // and then takes another GEMM kernel than the level batched over the whole matrix, so the two schedules agree to
-// round-off (bit for bit with MFGP_GEMM_TMA_MC=0, where every kernel sums k in the same order).
-// MFGP_OVERLAP_TRTRI=0 switches the overlap off.
+// round-off.
 int potrf_trtri_padded(mfgp_ctx* h, double* A, double* W, int npad, int nreal, cudaEvent_t ev_mid) {
-  static int overlap = -1;
-  if (overlap < 0) {
-    const char* e = getenv("MFGP_OVERLAP_TRTRI");
-    overlap = e ? (atoi(e) != 0) : 1;
-  }
   const int m = npad / LEAF;
   int rc;
-  potrf_env();
-  const bool la = USE_LA && h->s_hi && npad >= LA_MIN && npad <= la_nb(npad) * LA_MAXP && LA_TAIL == 0;
+  const bool la = h->s_hi && npad >= LA_MIN && npad <= la_nb(npad) * LA_MAXP;
   const int half = npad / 2;
-  if (!(overlap && la && h->s_mid && (m & (m - 1)) == 0 && npad >= 8192 && half % la_nb(npad) == 0)) {
+  if (!(la && h->s_mid && (m & (m - 1)) == 0 && npad >= 8192 && half % la_nb(npad) == 0)) {
     if ((rc = potrf_padded(h, A, W, npad, nreal))) return rc;
     if (ev_mid) CUDA_TRY(h, cudaEventRecord(ev_mid, h->stream));
     return trtri_padded(h, A, W, npad);
@@ -1192,7 +1071,7 @@ int lauum_padded(mfgp_ctx* h, const double* W, double* Kinv, int npad) {
 
 // T[i][c] = sum_{k<=i} W[i][k] * Ks[c][k]   (T: npad x cols_pad, row-major, ld = cols_pad)
 int trmm_store(mfgp_ctx* h, const double* W, int npad, const double* Ks, long long cols_pad, double* T) {
-  ARG_CHECK(h, npad % LEAF == 0 && cols_pad % dg::Big::BN == 0 && cols_pad < (1LL << 31));
+  ARG_CHECK(h, npad % LEAF == 0 && cols_pad % dg::Big16::BN == 0 && cols_pad < (1LL << 31));
   if (cols_pad == 0) return 0;
   dg::GemmParams p = gp(W, npad, Ks, npad, T, cols_pad, npad, (int)cols_pad, npad, 1.0, 0.0);
   p.ke_row = 1;
@@ -1208,7 +1087,7 @@ int syrk_tn_sub(mfgp_ctx* h, const double* T, long long ldt, int k, double* C, i
 }
 
 int trmm_right_store(mfgp_ctx* h, const double* L, int n, const double* E, long long ldc, double* Z) {
-  ARG_CHECK(h, n % LEAF == 0 && ldc % dg::Big::BN == 0 && ldc < (1LL << 31));
+  ARG_CHECK(h, n % LEAF == 0 && ldc % dg::Big16::BN == 0 && ldc < (1LL << 31));
   dg::GemmParams p = gp(L, n, E, ldc, Z, ldc, n, (int)ldc, n, 1.0, 0.0);
   p.ke_row = 1;
   return launch_gemm<true, false>(h, p, PC_MISC);
@@ -1216,9 +1095,10 @@ int trmm_right_store(mfgp_ctx* h, const double* L, int n, const double* E, long 
 
 int trmm_sumsq(mfgp_ctx* h, const double* W, int npad, const double* Ks, long long cols_pad,
                double* out_ss) {
-  ARG_CHECK(h, npad % LEAF == 0 && cols_pad % dg::Big::BN == 0);
+  ARG_CHECK(h, npad % LEAF == 0 && cols_pad % dg::Big16::BN == 0);
   if (cols_pad == 0) return 0;
-  if (trmm_tma_enabled() && cols_pad < (1LL << 31)) {
+  // TMA operands, measured r02: 2.42 -> 2.27 ms per 75 776 x 1024 launch, bit-identical sums
+  if (cols_pad < (1LL << 31)) {
     CUtensorMap tmW, tmK;
     if (make_map(&tmW, W, npad, npad, npad) && make_map(&tmK, Ks, npad, (unsigned long long)cols_pad, npad)) {
       prof_begin(h, PC_TRMM_SUMSQ);
@@ -1230,12 +1110,8 @@ int trmm_sumsq(mfgp_ctx* h, const double* W, int npad, const double* Ks, long lo
     }
   }
   prof_begin(h, PC_TRMM_SUMSQ);
-  if (tile_variant() == 16)
-    dg::trmm_sumsq_kernel<dg::Big16><<<(unsigned)(cols_pad / dg::Big16::BN), dg::Big16::THREADS,
-                                       dg::Big16::SMEM_BYTES, h->stream>>>(W, npad, Ks, out_ss);
-  else
-    dg::trmm_sumsq_kernel<dg::Big><<<(unsigned)(cols_pad / dg::Big::BN), dg::Big::THREADS,
-                                     dg::Big::SMEM_BYTES, h->stream>>>(W, npad, Ks, out_ss);
+  dg::trmm_sumsq_kernel<dg::Big16><<<(unsigned)(cols_pad / dg::Big16::BN), dg::Big16::THREADS,
+                                     dg::Big16::SMEM_BYTES, h->stream>>>(W, npad, Ks, out_ss);
   prof_end(h, PC_TRMM_SUMSQ);
   LAUNCH_CHECK(h);
   return 0;

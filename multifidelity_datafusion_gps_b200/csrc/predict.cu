@@ -4,7 +4,6 @@
 // src/abstractMFGP.py:104): the cross-covariance block is generated on the fly in column chunks
 // (never an N x M matrix in HBM beyond one chunk), the mean is reduced while it is generated, and
 // the variance comes from tmp = W Kx as a DMMA GEMM with a fused column sum-of-squares epilogue.
-#include <stdlib.h>
 #include "common.cuh"
 #include "fastmath.cuh"
 
@@ -1149,18 +1148,11 @@ int cross_gen_mc_launch(mfgp_ctx* h, const KParams& kp, const double* X, int N, 
   return 0;
 }
 
-int mc_small_applies(int N) {
-  static int enabled = -1;
-  if (enabled < 0) {
-    const char* e = getenv("MFGP_MC_SMALL");
-    enabled = e ? (atoi(e) != 0) : 1;
-  }
-  return enabled && N <= 64;
-}
+int mc_small_applies(int N) { return N <= 64; }
 
 // Fused generator + contraction for an upper level with N <= 64 (see mc_small_kernel).  Writes mu_c and the raw
 // column sums of squares of the npts * S columns; returns 0 without launching (and *took = 0) when the level does
-// not qualify.  MFGP_MC_SMALL=0 switches the path off.
+// not qualify.
 int mc_small_launch(mfgp_ctx* h, const KParams& kp, const double* X, int N, int npad, const double* W,
                     const double* alpha, const double* Xtest, const double* mu_l, const double* sd_l,
                     const double* eps, unsigned long long seed, long long m_global0, long long m_lo,

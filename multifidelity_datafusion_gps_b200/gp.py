@@ -11,7 +11,6 @@ SciPy's L-BFGS-B on the host, exactly as paramz does it; its objective is one GP
 No CPU fallback: constructing a model without a visible B200 raises ``MfgpError``.
 """
 import ctypes
-import os
 import re
 import threading
 
@@ -151,21 +150,6 @@ def to_device(arr, device):
 
 
 SMALL_BATCH_N = 128      # mfgp_lml_grad_batch: one CTA per hyper-parameter vector
-
-
-def _small_batch_enabled():
-    """MFGP_SMALL_BATCH=0 routes the optimiser's objective through mfgp_lml_grad (A/B and parity checks)."""
-    return os.environ.get("MFGP_SMALL_BATCH", "1") != "0"
-
-
-def _fast_lbfgsb_enabled():
-    """MFGP_FAST_LBFGSB=0: always go through scipy.optimize.fmin_l_bfgs_b's own Python wrapper."""
-    return os.environ.get("MFGP_FAST_LBFGSB", "1") != "0"
-
-
-def _lockstep_enabled():
-    """MFGP_LOCKSTEP=0: optimize_restarts runs its restarts one after the other (the reference's loop)."""
-    return os.environ.get("MFGP_LOCKSTEP", "1") != "0"
 
 
 class GPRegression:
@@ -396,7 +380,7 @@ class GPRegression:
         try:
             if not self._feasible(theta):
                 raise NotPositiveDefinite(0)
-            if getattr(self, "N", SMALL_BATCH_N + 1) <= SMALL_BATCH_N and _small_batch_enabled():
+            if getattr(self, "N", SMALL_BATCH_N + 1) <= SMALL_BATCH_N:
                 # the reference's own sizes: scalars-only kernel (no factors written; the posterior is
                 # rebuilt once, after the optimiser has finished)
                 lml_b, g_b, info = self.lml_and_grad_batch(theta[None, :], handle=self._opt_handle)
@@ -417,7 +401,7 @@ class GPRegression:
         """scipy.optimize.fmin_l_bfgs_b(fun, x0, maxfun=max_iters, maxiter=max_iters) as paramz's opt_lbfgsb
         calls it -- through the stepped driver around the same compiled routine when it reproduces SciPy's
         iterates bit for bit on this installation (_lbfgsb.selfcheck), else through SciPy's own wrapper."""
-        if _fast_lbfgsb_enabled() and _lbfgsb.selfcheck():
+        if _lbfgsb.selfcheck():
             return _lbfgsb.minimize(fun, x0, maxfun=max_iters, maxiter=max_iters)
         return _sopt.fmin_l_bfgs_b(fun, x0, maxfun=max_iters, maxiter=max_iters)
 
@@ -517,8 +501,10 @@ class GPRegression:
         return self
 
     def _lockstep_ok(self, n_runs):
+        # lock-step drives SciPy's compiled L-BFGS-B step directly; where that does not reproduce SciPy's own
+        # iterates (_lbfgsb.selfcheck) the restarts run one after the other, with the same results
         return (n_runs > 1 and getattr(self, "N", SMALL_BATCH_N + 1) <= SMALL_BATCH_N
-                and _small_batch_enabled() and _lockstep_enabled())
+                and _lbfgsb.selfcheck())
 
     def _objective_batch(self, thetas, free, handle=None):
         """[(objective, gradient over the free transformed parameters) or None] for full hyper-parameter
@@ -560,8 +546,6 @@ class GPRegression:
         but its own hyper-parameters, so every run follows exactly the trajectory it follows in the serial
         loop (same starts: run 0 from the current point, run i > 0 from starts[i], drawn by the caller in the
         serial order).  Returns [(index, objective at x_opt, x_opt)]."""
-        if not (_fast_lbfgsb_enabled() and _lbfgsb.selfcheck()):
-            return self._optimize_lockstep_threads(indices, starts, robust, max_iters)
         free = ~self._fixed
         nfree = int(free.sum())
         base = self.param_array.copy()
@@ -602,80 +586,6 @@ class GPRegression:
         final = self._objective_batch(thetas_of([runs[i].x for i in done]), free, handle=handle) if done else []
         return [(i, (v[0] if v is not None else np.inf), np.array(runs[i].x, dtype=np.float64))
                 for i, v in zip(done, final)]
-
-    def _optimize_lockstep_threads(self, indices, starts, robust, max_iters=1000):
-        """Fallback when SciPy's compiled step cannot be driven directly: every run is a
-        ``fmin_l_bfgs_b`` call in its own thread; their objective calls meet in a rendezvous and are
-        evaluated by one batched launch per round.  Same trajectories as the serial loop."""
-        free = ~self._fixed
-        nfree = int(free.sum())
-        base = self.param_array.copy()
-        handle = _ffi.get_handle(self.device)          # the calling thread's handle serves every batch
-        cv = threading.Condition()
-        pending, results, errors, finished = {}, {}, {}, {}
-        live = [len(indices)]
-
-        def flush():                                   # under cv, by the thread that completes the round
-            tids = sorted(pending)
-            thetas = [pending[t] for t in tids]
-            pending.clear()
-            try:
-                vals = self._objective_batch(thetas, free, handle=handle)
-            except BaseException as exc:               # a CUDA / argument failure fails every waiting run
-                vals = [exc] * len(tids)
-            results.update(zip(tids, vals))
-            cv.notify_all()
-
-        def evaluate(tid, theta):
-            with cv:
-                pending[tid] = theta
-                if len(pending) == live[0]:
-                    flush()
-                while tid not in results:
-                    cv.wait()
-                res = results.pop(tid)
-            if isinstance(res, BaseException):
-                raise res
-            return res
-
-        def retire():
-            with cv:
-                live[0] -= 1
-                if pending and len(pending) == live[0]:
-                    flush()
-
-        def run(i):
-            fails = [0]
-
-            def fun(x):
-                theta = base.copy()
-                theta[free] = logexp_f(x)
-                res = evaluate(i, theta)
-                if res is None:
-                    if fails[0] >= 10:
-                        raise NotPositiveDefinite(0)
-                    fails[0] += 1
-                    return np.inf, np.zeros(nfree)
-                fails[0] = 0
-                return res
-            try:
-                x0 = logexp_finv(base[free]) if starts[i] is None else logexp_finv(logexp_f(starts[i]))
-                x_opt, _, _ = _sopt.fmin_l_bfgs_b(fun, x0, maxfun=max_iters, maxiter=max_iters)
-                finished[i] = (i, fun(x_opt)[0], np.asarray(x_opt, dtype=np.float64))      # paramz: f_fp(x_opt)[0]
-            except BaseException as exc:
-                errors[i] = exc
-            finally:
-                retire()
-
-        threads = [threading.Thread(target=run, args=(i,), daemon=True) for i in indices]
-        for t in threads:
-            t.start()
-        for t in threads:
-            t.join()
-        self._dirty = True
-        if errors and not robust:
-            raise errors[min(errors)]
-        return [finished[i] for i in sorted(finished)]
 
     # -- prediction ----------------------------------------------------------------------------
     def level_struct(self):

@@ -735,16 +735,19 @@ def test_lockstep_restarts_equal_the_serial_loop(pkg, monkeypatch):
     """optimize_restarts (src/abstractMFGP.py:137) with the six restarts in lock-step on one GPU (one batched
     launch per round of evaluations) must end where the reference's serial loop ends: same runs, same
     objectives, same winner, bit for bit -- for the composite and the plain kernel."""
+    from multifidelity_datafusion_gps_b200 import gp
     _, X_hf, _ = _data(2, n_hf=14)
     for cls, args in ((pkg.GPDF, (2, 0.001, 2)), (pkg.NARGP, (2,))):
         out = {}
-        for mode in ("0", "1"):
-            monkeypatch.setenv("MFGP_LOCKSTEP", mode)
-            np.random.seed(3)
-            m = cls(*args, util.hf_2d, util.lf_2d)
-            m.fit(X_hf)
-            out[mode] = (m.hf_model.param_array.copy(), [f for _, f in m.hf_model.optimization_runs],
-                         [x.copy() for x, _ in m.hf_model.optimization_runs], m.predict(X_hf[:3]))
+        for mode in ("0", "1"):      # "0": the serial loop, "1": lock-step
+            with monkeypatch.context() as mp:
+                if mode == "0":
+                    mp.setattr(gp.GPRegression, "_lockstep_ok", lambda self, n: False)
+                np.random.seed(3)
+                m = cls(*args, util.hf_2d, util.lf_2d)
+                m.fit(X_hf)
+                out[mode] = (m.hf_model.param_array.copy(), [f for _, f in m.hf_model.optimization_runs],
+                             [x.copy() for x, _ in m.hf_model.optimization_runs], m.predict(X_hf[:3]))
         assert np.array_equal(out["0"][0], out["1"][0])
         assert out["0"][1] == out["1"][1] and len(out["1"][1]) == 7
         assert all(np.array_equal(a, b) for a, b in zip(out["0"][2], out["1"][2]))

@@ -1,6 +1,6 @@
 """Times one MC sweep at a small high-fidelity level (default N_h = 30, N_l = 100, M = 2^20, S = 100) and prints a
-fingerprint of the result; run once with MFGP_MC_SMALL=0 and once with the default to compare the fused small-level
-kernel (mc_small_kernel) with the general Ks + trmm_sumsq pair."""
+fingerprint of the result.  MFGP_PROBE_SAVE=<file.npy> keeps the result and MFGP_PROBE_COMPARE=<file.npy> compares
+with a kept one, so that two builds of the library (MFGP_LIB) can be set against each other."""
 import os
 import sys
 import time
@@ -29,9 +29,8 @@ for rep in range(3):
     mean, var, wsum = model.predict_mc_device(dX, S, None, 2, 0, dw)
     e_ev.record(); torch.cuda.synchronize()
     ms = s_ev.elapsed_time(e_ev)
-    print("N_h=%d N_l=%d M=%d S=%d MC_SMALL=%s rep %d: %.2f ms  %.1f M samples/s  pce_mean=%.15g  sum(var)=%.15g" %
-          (nh, nl, m, S, os.environ.get("MFGP_MC_SMALL", "default"), rep, ms, m * S / ms / 1e3, wsum,
-           float(var.sum().item())))
+    print("N_h=%d N_l=%d M=%d S=%d rep %d: %.2f ms  %.1f M samples/s  pce_mean=%.15g  sum(var)=%.15g" %
+          (nh, nl, m, S, rep, ms, m * S / ms / 1e3, wsum, float(var.sum().item())))
 out = os.environ.get("MFGP_PROBE_SAVE")
 if out:
     np.save(out, np.stack([mean.cpu().numpy(), var.cpu().numpy()]))
