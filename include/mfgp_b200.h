@@ -77,7 +77,8 @@ long long mfgp_launch_count(mfgp_handle_t h);
  * event pairs on the handle's stream (first 512 launches per class).  mfgp_profile_read synchronises
  * and returns, per class, the average launch duration in ms (h_ms[10]) and the launch count
  * (h_count[10]); classes: 0 assemble, 1 potrf leaf, 2 gemm (potrf/trtri), 3 solve, 4 lauum,
- * 5 grad_reduce, 6 cross-covariance, 7 trmm+sumsq, 8 misc, 9 argmax. */
+ * 5 grad_reduce, 6 cross-covariance, 7 trmm+sumsq, 8 misc, 9 argmax (the batch acquisition's fused update and
+ * arg-max stage). */
 int mfgp_profile_enable(mfgp_handle_t h, int on);
 int mfgp_profile_read(mfgp_handle_t h, double* h_ms, long long* h_count);
 
@@ -254,6 +255,33 @@ int mfgp_fill_normal(mfgp_handle_t h, unsigned long long seed, long long first, 
  * (src/adaptation_maximizers/scipydirect_wrapper.py:22-26) by a candidate-set argmax:
  * h_val[0] = max_i v[i], h_idx[0] = lowest i attaining it (np.argmax semantics). */
 int mfgp_argmax(mfgp_handle_t h, const double* d_v, long long C, double* h_val, long long* h_idx);
+
+/* K8b -- greedy batch acquisition: q high-fidelity points per adaptation step instead of one
+ * (src/abstractMFGP.py:317-359 acquires one per step and refits).  At fixed theta the predictive variance does not
+ * depend on the targets, so the q points that q sequential steps (arg-max, append at fixed theta) would pick are a
+ * pivoted partial Cholesky of the posterior covariance over the candidate set:
+ *   v_0(c) = k(c, c) - |W k_c|^2 (unclipped),  s^2 = noise + 1e-8 + jitter (the diagonal mfgp_append_point adds),
+ *   pick p_i = argmax_c max(v_i(c), 1e-15) (+ noise), lowest index on ties,
+ *   R[i][c] = (k(c, a_i) - k_c^T K_y^-1 k(X, a_i) - sum_{l<i} R[l][c] R[l][p_i]) / sqrt(v_i(p_i) + s^2),
+ *   v_{i+1}(c) = v_i(c) - R[i][c]^2,   a_i = d_cands[p_i] (augmented row).
+ * Step-wise protocol, so that the same calls serve one GPU and candidates sharded over ranks:
+ *   _begin computes v_0 (the pass mfgp_predict makes) and returns the LOCAL winner of pick 0;
+ *   _step(i) conditions on pick i, given by its record h_rec_in (the GLOBAL winner's; on one GPU the record the
+ *   previous call returned), and returns the local winner of pick i + 1.
+ * Record (1 + D + q doubles): [v_i(p) unclipped, a (D values), R[0..i)[p], zeros].  h_val[0] = the winner's reported
+ * variance max(v, 1e-15) (+ noise), h_idx[0] = its index in [0, C).  One synchronisation per call.
+ * 1 <= q <= MFGP_ACQ_MAX_Q, C >= 1, 0 <= i < q.  jitter: the level's factorisation jitter.  d_ws (at least
+ * mfgp_acq_batch_ws_bytes(N, C, q), of which the part beyond the fixed regions holds the prediction chunk) carries
+ * state from call to call and must not be touched between the calls of one batch.
+ * _step returns i + 1 (LAPACK-style) if v_i(p_i) + s^2 <= 0. */
+#define MFGP_ACQ_MAX_Q 64
+size_t mfgp_acq_batch_ws_bytes(int N, long long C, int q);
+int mfgp_acq_batch_begin(mfgp_handle_t h, const mfgp_level_t* gp, const double* d_cands, long long C, int q,
+                         int include_noise, double* d_ws, size_t ws_bytes, double* h_val, long long* h_idx,
+                         double* h_rec);
+int mfgp_acq_batch_step(mfgp_handle_t h, const mfgp_level_t* gp, const double* d_cands, long long C, int q,
+                        int include_noise, double jitter, int i, const double* h_rec_in, double* d_ws,
+                        size_t ws_bytes, double* h_val, long long* h_idx, double* h_rec);
 
 /* K9 -- polynomial-chaos projection on a quadrature grid (SURVEY.md section 8f rank 2).  Replaces
  * cp.fit_quadrature / cp.E / cp.Var as src/gpc/chaospy_wrapper.py:18-29 uses them, for independent

@@ -13,6 +13,7 @@ Extensions (keyword-only, defaults reproduce the reference):
   reference, which collapses the LF level to its mean, src/abstractMFGP.py:104).
 * ``acquisition_argmax``  candidate-set arg-max of the predictive variance (used by
   ``CandidateSetMaximizer``), optionally sharded over ranks.
+* ``acquisition_batch``  greedy batch of q candidates per adaptation step (``adapt_batch_size``).
 * ``broadcast_state``  NCCL broadcast of the fitted state so that other ranks can predict.
 """
 import ctypes
@@ -84,6 +85,18 @@ class MultifidelityDataFusion(AbstractMFGP):
         self.hf_X = new_hf_X
         self.hf_Y = np.vstack((self.hf_Y, y))
         self.hf_model.append_point(self.__augment_Data(x), y)
+
+    def _append_hf_points(self, new_hf_X, k):
+        """The last k rows of new_hf_X (one acquired batch) join the high-fidelity GP at fixed hyper-parameters:
+        f_exact is called ONCE on the (k, d) block -- the expensive simulations of a batch run together -- and the
+        rows then enter by bordered updates, in order."""
+        X = np.atleast_2d(new_hf_X[len(new_hf_X) - k:])
+        Y = np.asarray(self.f_exact(X), dtype=np.float64).reshape(k, 1)
+        self.hf_X = new_hf_X
+        self.hf_Y = np.vstack((self.hf_Y, Y))
+        Xa = self.__augment_Data(X)
+        for j in range(k):
+            self.hf_model.append_point(Xa[j:j + 1], Y[j:j + 1])
 
     # -- A10 adapt --------------------------------------------------------------------------------
     def adapt(self, adapt_steps: int, plot_mode: str = None, X_test: np.ndarray = None,
@@ -466,6 +479,57 @@ class MultifidelityDataFusion(AbstractMFGP):
         if distributed and world > 1:
             val, idx = dist.gather_argmax(val, idx, device="cuda:%d" % self.device)
         return int(idx), float(val)
+
+    def acquisition_batch(self, candidates, q, distributed=False, cache=True):
+        """Greedy batch of q candidates for one adaptation step: (indices (q,) int64, variances (q,)).  Pick i is the
+        arg-max of the predictive variance given the training set plus picks 0..i-1 as noisy observations at the
+        current hyper-parameters -- the points q sequential ``acquisition_argmax`` + ``append_point`` steps pick,
+        computed without the targets (mfgp_acq_batch_*, a pivoted partial Cholesky of the posterior covariance over
+        the candidates).  variances[i] includes the noise, as GPy reports it; pick 0 is ``acquisition_argmax``.
+        distributed / cache: as in acquisition_argmax; per pick the ranks agree on the winner with one all_gather
+        and its owner broadcasts the pivot record (1 + D + q doubles)."""
+        C = int(candidates.shape[0])
+        q = int(q)
+        if not 1 <= q <= min(_ffi.ACQ_MAX_Q, C):
+            raise ValueError("batch size q = %d must lie in [1, min(%d, number of candidates = %d)]"
+                             % (q, _ffi.ACQ_MAX_Q, C))
+        rank, world = dist.rank_world() if distributed else (0, 1)
+        lo, hi = dist.shard_range(C, rank, world)
+        self._apply_add_noise()
+        hf = self.hf_model
+        lvl = hf.level_struct()
+        D = hf.D
+        jitter = float(hf.last_jitter)
+        h = _ffi.get_handle(self.device)
+        if hi > lo:
+            dXa = self._resident_candidates(candidates, lo, hi) if cache else self._augment_host_input(candidates[lo:hi])
+            ws = gp.workspace(self.device, h.lib.mfgp_acq_batch_ws_bytes(hf.N, hi - lo, q))
+        indices = np.empty(q, dtype=np.int64)
+        variances = np.empty(q)
+        rec = np.zeros(1 + D + q)
+        c_val, c_idx = ctypes.c_double(), ctypes.c_longlong()
+        for i in range(q):
+            val, idx, local = -np.inf, -1, np.zeros(1 + D + q)
+            if hi > lo:
+                if i == 0:
+                    rc = h.lib.mfgp_acq_batch_begin(h.h, ctypes.byref(lvl), dXa.data_ptr(), hi - lo, q, 1,
+                                                    ws.data_ptr(), ws.numel() * 8, ctypes.byref(c_val),
+                                                    ctypes.byref(c_idx), local.ctypes.data)
+                else:
+                    rc = h.lib.mfgp_acq_batch_step(h.h, ctypes.byref(lvl), dXa.data_ptr(), hi - lo, q, 1, jitter,
+                                                   i - 1, rec.ctypes.data, ws.data_ptr(), ws.numel() * 8,
+                                                   ctypes.byref(c_val), ctypes.byref(c_idx), local.ctypes.data)
+                h.check(rc)
+                val, idx = c_val.value, lo + c_idx.value
+            elif i > 0 and not rec[0] + hf.likelihood.variance + 1e-8 + jitter > 0.0:
+                raise _ffi.NotPositiveDefinite(i)          # what the ranks holding candidates report for this pick
+            if distributed and world > 1:
+                val, idx = dist.gather_argmax(val, idx, device="cuda:%d" % self.device)
+                rec = dist.broadcast_record(local, dist.shard_owner(idx, C, world), device="cuda:%d" % self.device)
+            else:
+                rec = local
+            indices[i], variances[i] = idx, val
+        return indices, variances
 
     # -- multi-GPU state ------------------------------------------------------------------------------
     def broadcast_state(self, src=0):

@@ -20,9 +20,15 @@ from .adaptation_maximizers import AbstractMaximizer
 class AbstractMFGP(metaclass=abc.ABCMeta):
     parallel_restarts = False     # set True to spread optimize_restarts over the ranks (SURVEY.md 8f rank 1)
     refit_every = 1               # adaptation steps per hyper-parameter refit (SURVEY.md 8f rank 3)
+    adapt_batch_size = 1          # high-fidelity points acquired per adaptation step (adapt_maximizer.maximize_batch)
 
     def _append_hf_point(self, new_hf_X):
         """One acquired point at fixed hyper-parameters; models without an incremental path refit."""
+        self.fit(new_hf_X)
+
+    def _append_hf_points(self, new_hf_X, k):
+        """The last k rows of new_hf_X (one acquired batch) at fixed hyper-parameters; models without an
+        incremental path refit."""
         self.fit(new_hf_X)
 
     @abc.abstractmethod
@@ -117,9 +123,12 @@ class AbstractMFGP(metaclass=abc.ABCMeta):
                        plot_error: bool = False, eps: float = 1e-8):
         """The loop body of the reference's adapt_and_plot with the drawing removed: acquire the most
         uncertain input, append it, refit; stop early once |fopt| < eps.  With plot_error the test
-        MSE before each refit is recorded in ``self.mse_history`` (what the reference plots)."""
+        MSE before each refit is recorded in ``self.mse_history`` (what the reference plots).
+        With ``adapt_batch_size`` > 1 every step acquires a batch instead (_adapt_batches)."""
         self.mse_history = []
         self.acquired_points = []
+        if int(getattr(self, "adapt_batch_size", 1)) > 1:
+            return self._adapt_batches(plot_error or plot_uncertainties)
         for i in range(self.adapt_steps):
             acquired_x, fopt = self.get_input_with_highest_uncertainty(self)
             self.acquired_points.append((np.array(acquired_x, dtype=np.float64), float(np.ravel(fopt)[0])))
@@ -137,4 +146,33 @@ class AbstractMFGP(metaclass=abc.ABCMeta):
                 self.adapt_steps = i + 1
                 print("Iteration stopped after {} iterations!".format(i + 1)
                       + " minimum uncertainty reached: {:e}".format(float(np.ravel(fopt)[0])))
+                break
+
+    def _adapt_batches(self, record_mse):
+        """adapt_and_plot with q = adapt_batch_size points per step: the maximiser's greedy batch (the points q
+        sequential steps at fixed hyper-parameters would pick), cut after the first point with |fopt| < eps -- the
+        sequential loop stops after acquiring that point -- then one refit on a refit step, or else one f_exact
+        call on the block and bordered updates.  Every point goes into ``acquired_points``; the test MSE is
+        recorded once per step."""
+        q = int(self.adapt_batch_size)
+        for i in range(self.adapt_steps):
+            X_new, fopt = self.adapt_maximizer.maximize_batch(self.predict, self.lower_bound, self.upper_bound, q)
+            X_new = np.atleast_2d(np.asarray(X_new, dtype=np.float64))
+            fopt = np.ravel(np.asarray(fopt, dtype=np.float64))
+            small = np.flatnonzero(np.abs(fopt) < self.eps)
+            k = int(small[0]) + 1 if small.size else len(fopt)
+            X_new = X_new[:k]
+            for j in range(k):
+                self.acquired_points.append((X_new[j].copy(), float(fopt[j])))
+            new_hf_X = np.vstack((self.hf_X, X_new))
+            if record_mse and self.X_test is not None and self.Y_test is not None:
+                self.mse_history.append(self.get_mse(self.X_test, self.Y_test))
+            if (i + 1) % max(1, int(getattr(self, "refit_every", 1))) == 0:
+                self.fit(new_hf_X)
+            else:
+                self._append_hf_points(new_hf_X, k)
+            if small.size:
+                self.adapt_steps = i + 1
+                print("Iteration stopped after {} iterations!".format(i + 1)
+                      + " minimum uncertainty reached: {:e}".format(float(fopt[k - 1])))
                 break

@@ -4,7 +4,8 @@ The reference's maximizers run a sequential DIRECT search of up to 20 000 single
 calls (src/adaptation_maximizers/scipydirect_wrapper.py:22-26).  This maximizer scores a whole
 candidate set in one batched GPU predict and takes the arg-max on the device (K8); with
 ``torch.distributed`` initialised the candidates are split contiguously over the ranks and the
-per-rank winners are combined with one all_gather (max value, lowest global index)."""
+per-rank winners are combined with one all_gather (max value, lowest global index).  ``maximize_batch``
+takes a greedy batch of q candidates per step through the owner's ``acquisition_batch``."""
 import numpy as np
 
 from .abstract_maximizer import AbstractMaximizer
@@ -18,6 +19,7 @@ class CandidateSetMaximizer(AbstractMaximizer):
         self.seed = seed
         self.distributed = distributed
         self.last_index = None
+        self.last_indices = None
         self.last_gap = None
 
     def _candidates(self, lower_bound, upper_bound):
@@ -40,3 +42,13 @@ class CandidateSetMaximizer(AbstractMaximizer):
             val = float(var[idx])
         self.last_index = idx
         return cands[idx].copy(), -val
+
+    def maximize_batch(self, model_predict: callable, lower_bound: np.ndarray, upper_bound: np.ndarray, q: int):
+        owner = getattr(model_predict, "__self__", None)
+        if int(q) == 1 or owner is None or not hasattr(owner, "acquisition_batch"):
+            return super().maximize_batch(model_predict, lower_bound, upper_bound, q)
+        cands = self._candidates(lower_bound, upper_bound)
+        idx, var = owner.acquisition_batch(cands, int(q), distributed=self.distributed)   # GPU K6 + K8b
+        self.last_indices = idx
+        self.last_index = int(idx[-1])
+        return cands[idx].copy(), -var

@@ -10,7 +10,14 @@ int cross_gen_launch(mfgp_ctx* h, const KParams& kp, const double* X, int N, int
                      const double* alpha, const double* Xq, long long ncols, long long cols_pad,
                      double* Ks, double* mean);
 int finish_var_launch(mfgp_ctx* h, const double* ss, long long n, double kdiag, double noise_add,
-                      double* var);
+                      double* var, bool latent = false);
+int acq_partials_doubles();
+int kinv_apply_launch(mfgp_ctx* h, const double* W, int npad, int N, const double* k, double* l_tmp, double* u);
+int acq_coef_launch(mfgp_ctx* h, const double* u, int N, int npad1, double* coef);
+int acq_update_launch(mfgp_ctx* h, const double* kg, double* R, long long C, int i, const double* rp, double rho,
+                      double* v, double noise_add, double* partials, double* best);
+int acq_gather_launch(mfgp_ctx* h, const double* best, const double* v, const double* cands, int D,
+                      const double* R, long long C, int nr, int q, double* out);
 int build_locs_launch(mfgp_ctx* h, const double* X, long long rows, int d, const double* d_offs,
                       int E, double tau, double* out);
 int concat_aug_launch(mfgp_ctx* h, const double* X, const double* vals, long long rows, int d, int E,
@@ -543,9 +550,10 @@ static long long whole_waves(long long cols) {
   return cols > wave ? cols / wave * wave : cols;
 }
 
+// latent: d_var receives k(x, x) - |W k_x|^2 unclipped and without noise (the batch acquisition's v_0)
 static int predict_impl(mfgp_ctx* h, const mfgp_level_t* gp, const KParams& kp, const double* d_Xnew,
                         long long M, double* d_mean, double* d_var, int include_noise, double* d_ws,
-                        size_t ws_bytes) {
+                        size_t ws_bytes, bool latent = false) {
   const int npad = mfgp_padded_n(gp->N);
   int rc;
   if (M <= 0) return 0;
@@ -566,7 +574,7 @@ static int predict_impl(mfgp_ctx* h, const mfgp_level_t* gp, const KParams& kp, 
                                cols_pad, Ks, d_mean ? d_mean + c0 : nullptr)))
       return rc;
     if ((rc = trmm_sumsq(h, gp->d_W, npad, Ks, cols_pad, ss))) return rc;
-    if ((rc = finish_var_launch(h, ss, ncols, kp.kdiag, include_noise ? kp.noise : 0.0, d_var + c0)))
+    if ((rc = finish_var_launch(h, ss, ncols, kp.kdiag, include_noise ? kp.noise : 0.0, d_var + c0, latent)))
       return rc;
   }
   return 0;
@@ -1100,6 +1108,130 @@ int mfgp_argmax(mfgp_handle_t h, const double* d_v, long long C, double* h_val, 
   h_val[0] = h->h_pinned[16];
   memcpy(h_idx, h->h_pinned + 17, sizeof(long long));
   return 0;
+}
+
+// ---- K8b greedy batch acquisition (math: predict.cu, acq_update_kernel) -----------------------------------------
+// Scratch layout in the caller's d_ws, every region on a 128-double boundary: v (C) | kg (C) | R (q, C) |
+// X' = [X; a] ((N+1) x MFGP_MAX_D) | k(X, a), W k, u / coefficients (Npad(N+1) each) | pivot record (128) |
+// arg-max partials | winner (2) | the prediction chunk for v_0 (the rest).  v and R carry over from call to call.
+struct AcqLayout {
+  double *v, *kg, *R, *Xp, *krow, *l, *coef, *rec, *partials, *best, *chunk;
+  long long chunk_doubles;
+};
+
+static long long acq_fixed_doubles(int N, long long C, int q, AcqLayout* L, double* base) {
+  const long long np1 = mfgp_padded_n(N + 1);
+  long long off = 0;
+  auto take = [&](long long n) {
+    double* p = base ? base + off : nullptr;
+    off += (n + 127) / 128 * 128;
+    return p;
+  };
+  double* v = take(C);
+  double* kg = take(C);
+  double* R = take((long long)q * C);
+  double* Xp = take((long long)(N + 1) * MFGP_MAX_D);
+  double* krow = take(np1);
+  double* l = take(np1);
+  double* coef = take(np1);
+  double* rec = take(128);
+  double* partials = take(acq_partials_doubles());
+  double* best = take(2);
+  if (L) *L = AcqLayout{v, kg, R, Xp, krow, l, coef, rec, partials, best, base ? base + off : nullptr, 0};
+  return off;
+}
+
+static int acq_prepare(mfgp_ctx* h, const mfgp_level_t* gp, const double* d_cands, long long C, int q,
+                       double* d_ws, size_t ws_bytes, const double* h_val, const long long* h_idx,
+                       const double* h_rec, KParams* kp, AcqLayout* L) {
+  int rc = level_kparams(h, gp, kp);
+  if (rc) return rc;
+  ARG_CHECK(h, gp->d_W != nullptr && d_cands && d_ws && h_val && h_idx && h_rec);
+  ARG_CHECK(h, C >= 1 && q >= 1 && q <= MFGP_ACQ_MAX_Q);
+  const long long fixed = acq_fixed_doubles(gp->N, C, q, L, d_ws);
+  const long long have = (long long)(ws_bytes / sizeof(double));
+  ARG_CHECK(h, have >= fixed);
+  L->chunk_doubles = have - fixed;
+  return 0;
+}
+
+// one synchronisation: the winner's value, index and record arrive through mapped pinned memory
+static int acq_finish(mfgp_ctx* h, const AcqLayout& L, const double* d_cands, int D, long long C, int nr, int q,
+                      double* h_val, long long* h_idx, double* h_rec) {
+  int rc = acq_gather_launch(h, L.best, L.v, d_cands, D, L.R, C, nr, q, h->d_batch + 128);
+  if (rc) return rc;
+  CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+  const double* out = h->h_batch + 128;
+  long long idx;
+  memcpy(&idx, out + 1, sizeof(idx));
+  if (idx < 0) {
+    snprintf(h->err, sizeof(h->err), "batch acquisition: no candidate has a comparable variance (NaN)");
+    return -1;
+  }
+  h_val[0] = out[0];
+  h_idx[0] = idx;
+  memcpy(h_rec, out + 2, (size_t)(1 + D + q) * sizeof(double));
+  return 0;
+}
+
+size_t mfgp_acq_batch_ws_bytes(int N, long long C, int q) {
+  if (N < 1 || C < 1 || q < 1 || q > MFGP_ACQ_MAX_Q) return 0;
+  size_t chunk = mfgp_predict_ws_bytes(N, C);          // what mfgp_predict's callers size for C rows, capped
+  if (chunk > ((size_t)1 << 30)) chunk = (size_t)1 << 30;
+  const size_t least = mfgp_predict_ws_bytes(N, 128);
+  if (chunk < least) chunk = least;
+  return (size_t)acq_fixed_doubles(N, C, q, nullptr, nullptr) * sizeof(double) + chunk;
+}
+
+int mfgp_acq_batch_begin(mfgp_handle_t h, const mfgp_level_t* gp, const double* d_cands, long long C, int q,
+                         int include_noise, double* d_ws, size_t ws_bytes, double* h_val, long long* h_idx,
+                         double* h_rec) {
+  ENTER(h);
+  KParams kp;
+  AcqLayout L;
+  int rc = acq_prepare(h, gp, d_cands, C, q, d_ws, ws_bytes, h_val, h_idx, h_rec, &kp, &L);
+  if (rc) return rc;
+  // v_0 through mfgp_predict's own chunk loop (same generator, same DMMA contraction, kg as the mean's scratch),
+  // finished latent: the clip and the noise are applied only where values are reported or compared
+  if ((rc = predict_impl(h, gp, kp, d_cands, C, L.kg, L.v, 0, L.chunk, (size_t)L.chunk_doubles * sizeof(double),
+                         true)))
+    return rc;
+  if ((rc = acq_update_launch(h, nullptr, L.R, C, 0, nullptr, 1.0, L.v, include_noise ? kp.noise : 0.0, L.partials,
+                              L.best)))
+    return rc;
+  return acq_finish(h, L, d_cands, gp->D, C, 0, q, h_val, h_idx, h_rec);
+}
+
+int mfgp_acq_batch_step(mfgp_handle_t h, const mfgp_level_t* gp, const double* d_cands, long long C, int q,
+                        int include_noise, double jitter, int i, const double* h_rec_in, double* d_ws,
+                        size_t ws_bytes, double* h_val, long long* h_idx, double* h_rec) {
+  ENTER(h);
+  KParams kp;
+  AcqLayout L;
+  int rc = acq_prepare(h, gp, d_cands, C, q, d_ws, ws_bytes, h_val, h_idx, h_rec, &kp, &L);
+  if (rc) return rc;
+  ARG_CHECK(h, h_rec_in && i >= 0 && i < q);
+  const int N = gp->N, D = gp->D;
+  const int npad = mfgp_padded_n(N), npad1 = mfgp_padded_n(N + 1);
+  const double rho2 = h_rec_in[0] + kp.noise + JITTER_CONST + jitter;   // v_i(p_i) + s^2
+  if (!(rho2 > 0.0)) return i + 1;
+  // the pivot's record (a, R[0..i)[p]) to the device through the pinned staging block
+  const int nrec = 1 + D + q;
+  memcpy(h->h_batch, h_rec_in, (size_t)nrec * sizeof(double));
+  CUDA_TRY(h, cudaMemcpyAsync(L.rec, h->h_batch, (size_t)nrec * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+  CUDA_TRY(h, cudaMemcpyAsync(L.Xp, gp->d_X, (size_t)N * D * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
+  CUDA_TRY(h, cudaMemcpyAsync(L.Xp + (long long)N * D, L.rec + 1, (size_t)D * sizeof(double),
+                              cudaMemcpyDeviceToDevice, h->stream));
+  // u = K_y^-1 k(X, a), then k(c, a) - k_c^T u for every candidate in one mean-mode pass over X' = [X; a]
+  if ((rc = cross_gen_launch(h, kp, gp->d_X, N, npad, gp->d_alpha, L.Xp + (long long)N * D, 1, 1, L.krow, nullptr)))
+    return rc;
+  if ((rc = kinv_apply_launch(h, gp->d_W, npad, N, L.krow, L.l, L.coef))) return rc;
+  if ((rc = acq_coef_launch(h, L.coef, N, npad1, L.coef))) return rc;
+  if ((rc = cross_gen_launch(h, kp, L.Xp, N + 1, npad1, L.coef, d_cands, C, C, nullptr, L.kg))) return rc;
+  if ((rc = acq_update_launch(h, L.kg, L.R, C, i, L.rec + 1 + D, sqrt(rho2), L.v, include_noise ? kp.noise : 0.0,
+                              L.partials, L.best)))
+    return rc;
+  return acq_finish(h, L, d_cands, D, C, i + 1, q, h_val, h_idx, h_rec);
 }
 
 }  // extern "C"

@@ -106,12 +106,13 @@ __global__ void __launch_bounds__(256)
   if (lane == 0 && mean) mean[c] = acc;
 }
 
+// floor = 1e-15 for GPy's reported variance; -inf leaves the latent variance unclipped (batch acquisition)
 __global__ void finish_var_kernel(const double* ss, long long n, double kdiag, double noise_add,
-                                  double* var) {   // may run in place (ss == var)
+                                  double floor, double* var) {   // may run in place (ss == var)
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   double v = kdiag - ss[i];
-  v = v < 1e-15 ? 1e-15 : v;   // GPy posterior.py: np.clip(var, 1e-15, inf)
+  v = v < floor ? floor : v;   // GPy posterior.py: np.clip(var, 1e-15, inf)
   var[i] = v + noise_add;
 }
 
@@ -919,6 +920,93 @@ __global__ void argmax_stage2_kernel(const double* __restrict__ pval, const long
   }
 }
 
+// ---- K8b greedy batch acquisition: pivoted partial Cholesky of the posterior covariance over the candidates ----
+// At fixed theta the posterior covariance kappa(c, a) = k(c, a) - k_c^T K_y^-1 k_a does not depend on the targets,
+// so the q points that q sequential "arg-max, then append" steps pick are known in advance.  With
+// s^2 = noise + 1e-8 + jitter (the diagonal of a bordered update) and v_0(c) = k(c, c) - |W k_c|^2 (unclipped),
+// step i conditions on pivot p_i with augmented row a_i:
+//   u_i = K_y^-1 k(X, a_i),   g_i(c) = sum_k K(c, X_k) u_i[k],   rho_i = sqrt(v_i(p_i) + s^2),
+//   R[i][c] = (k(c, a_i) - g_i(c) - sum_{l<i} R[l][c] R[l][p_i]) / rho_i,   v_{i+1}(c) = v_i(c) - R[i][c]^2.
+// k(c, a_i) - g_i(c) comes from ONE mean-mode pass of the cross-covariance generator over X' = [X; a_i] with the
+// coefficients [-u_i; 1] (acq_coef_kernel): no C x N block is stored.  Reported and compared values are GPy's
+// max(v, 1e-15) + noise, lowest index on ties, so the first pick is exactly mfgp_argmax over mfgp_predict's variance.
+
+// coef[k] = -u[k] (k < N), 1 (k == N), 0 on the pad up to npad1
+__global__ void acq_coef_kernel(const double* u, int N, int npad1, double* coef) {   // may run in place
+  const int k = blockIdx.x * blockDim.x + threadIdx.x;
+  if (k < npad1) coef[k] = k < N ? -u[k] : (k == N ? 1.0 : 0.0);
+}
+
+// Per candidate (grid-stride): with kg, r = (kg[c] - sum_{l<i} R[l][c] rp[l]) / rho in a fixed order, R[i][c] = r,
+// v[c] -= r^2; without kg, v is read as it is (the first pick).  Then stage 1 of the arg-max over
+// max(v, 1e-15) + noise_add with argmax_stage1_kernel's tie rule; argmax_stage2_kernel finishes it.
+// R is (q, C) row-major: the reads of one l are coalesced over the candidates.
+__global__ void __launch_bounds__(256)
+    acq_update_kernel(const double* __restrict__ kg, double* __restrict__ R, long long C, int i,
+                      const double* __restrict__ rp, double rho, double* __restrict__ v, double noise_add,
+                      double* __restrict__ pval, long long* __restrict__ pidx) {
+  __shared__ double srp[MFGP_ACQ_MAX_Q];
+  __shared__ double sv[256];
+  __shared__ long long si[256];
+  if (kg)
+    for (int l = threadIdx.x; l < i; l += blockDim.x) srp[l] = rp[l];
+  __syncthreads();
+  double best = -INFINITY;
+  long long bi = 0x7fffffffffffffffLL;
+  for (long long c = (long long)blockIdx.x * blockDim.x + threadIdx.x; c < C;
+       c += (long long)gridDim.x * blockDim.x) {
+    double x = v[c];
+    if (kg) {
+      double t = kg[c];
+      for (int l = 0; l < i; l++) t = fma(-R[(long long)l * C + c], srp[l], t);
+      const double r = t / rho;
+      R[(long long)i * C + c] = r;
+      x = fma(-r, r, x);
+      v[c] = x;
+    }
+    const double rep = (x < 1e-15 ? 1e-15 : x) + noise_add;   // what finish_var_kernel reports
+    if (rep > best) {   // strictly greater: the lowest index wins (indices ascend per thread)
+      best = rep;
+      bi = c;
+    }
+  }
+  sv[threadIdx.x] = best;
+  si[threadIdx.x] = bi;
+  __syncthreads();
+  for (int o = 128; o > 0; o >>= 1) {
+    if (threadIdx.x < o) {
+      double x = sv[threadIdx.x + o];
+      long long xi = si[threadIdx.x + o];
+      if (x > sv[threadIdx.x] || (x == sv[threadIdx.x] && xi < si[threadIdx.x])) {
+        sv[threadIdx.x] = x;
+        si[threadIdx.x] = xi;
+      }
+    }
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) {
+    pval[blockIdx.x] = sv[0];
+    pidx[blockIdx.x] = si[0];
+  }
+}
+
+// The winner's record for the host (out: mapped pinned memory): out[0] = reported variance, out[1] = local index
+// (int64 bits), out[2..] = [v(p) unclipped, a = cands[p] (D values), R[0..nr)[p], zeros up to q entries].
+__global__ void acq_gather_kernel(const double* __restrict__ best_val, const long long* __restrict__ best_idx,
+                                  const double* __restrict__ v, const double* __restrict__ cands, int D,
+                                  const double* __restrict__ R, long long C, int nr, int q, double* __restrict__ out) {
+  const long long p = best_idx[0];
+  const bool ok = p >= 0 && p < C;   // no candidate with a comparable variance (all NaN): the host reports it
+  double* rec = out + 2;
+  if (threadIdx.x == 0) {
+    out[0] = best_val[0];
+    out[1] = __longlong_as_double(ok ? p : -1LL);
+    rec[0] = ok ? v[p] : NAN;
+  }
+  for (int k = threadIdx.x; k < D; k += blockDim.x) rec[1 + k] = ok ? cands[p * D + k] : NAN;
+  for (int l = threadIdx.x; l < q; l += blockDim.x) rec[1 + D + l] = ok && l < nr ? R[(long long)l * C + p] : 0.0;
+}
+
 // sum_i w[i]*x[i], two deterministic stages
 __global__ void __launch_bounds__(256)
     wdot_stage1_kernel(const double* __restrict__ w, const double* __restrict__ x, long long n,
@@ -1085,13 +1173,13 @@ int solve_alpha_launch(mfgp_ctx* h, const double* L, const double* W, int npad, 
 }
 
 
+int kinv_apply_launch(mfgp_ctx* h, const double* W, int npad, int N, const double* k, double* l_tmp, double* u);
+
 // l = W k and t = W^T l for the bordered update, then the finishing kernel
 int append_point_launch(mfgp_ctx* h, const double* k, int N, int npad, double kaa, double* A, double* W,
                         int write_L, double* l_tmp, double* t_tmp, double* d_out2) {
-  trmv_lower_kernel<<<nblk(npad, 8), 256, 0, h->stream>>>(W, npad, k, N, l_tmp);
-  LAUNCH_CHECK(h);
-  trmv_lower_t_kernel<<<npad / 32, 256, 0, h->stream>>>(W, npad, l_tmp, t_tmp);
-  LAUNCH_CHECK(h);
+  int rc = kinv_apply_launch(h, W, npad, N, k, l_tmp, t_tmp);
+  if (rc) return rc;
   append_finish_kernel<<<1, 256, 0, h->stream>>>(l_tmp, t_tmp, N, npad, kaa, A, W, write_L, h->d_info, d_out2);
   LAUNCH_CHECK(h);
   return 0;
@@ -1192,9 +1280,9 @@ int predict_configure(mfgp_ctx* h) {
 }
 
 int finish_var_launch(mfgp_ctx* h, const double* ss, long long n, double kdiag, double noise_add,
-                      double* var) {
+                      double* var, bool latent) {
   if (n <= 0) return 0;
-  finish_var_kernel<<<nblk(n, 256), 256, 0, h->stream>>>(ss, n, kdiag, noise_add, var);
+  finish_var_kernel<<<nblk(n, 256), 256, 0, h->stream>>>(ss, n, kdiag, noise_add, latent ? -INFINITY : 1e-15, var);
   LAUNCH_CHECK(h);
   return 0;
 }
@@ -1305,6 +1393,47 @@ int argmax_launch(mfgp_ctx* h, const double* v, long long n, double* d_val, long
   argmax_stage1_kernel<<<nb, 256, 0, h->stream>>>(v, n, pval, pidx);
   LAUNCH_CHECK(h);
   argmax_stage2_kernel<<<1, 256, 0, h->stream>>>(pval, pidx, nb, d_val, d_idx);
+  LAUNCH_CHECK(h);
+  return 0;
+}
+
+int acq_partials_doubles() { return 2 * RED_BLOCKS; }
+
+// u = K_y^-1 k = W^T (W k) for one column k (zero on the pad); l_tmp, u: npad doubles
+int kinv_apply_launch(mfgp_ctx* h, const double* W, int npad, int N, const double* k, double* l_tmp, double* u) {
+  trmv_lower_kernel<<<nblk(npad, 8), 256, 0, h->stream>>>(W, npad, k, N, l_tmp);
+  LAUNCH_CHECK(h);
+  trmv_lower_t_kernel<<<npad / 32, 256, 0, h->stream>>>(W, npad, l_tmp, u);
+  LAUNCH_CHECK(h);
+  return 0;
+}
+
+int acq_coef_launch(mfgp_ctx* h, const double* u, int N, int npad1, double* coef) {
+  acq_coef_kernel<<<nblk(npad1, 256), 256, 0, h->stream>>>(u, N, npad1, coef);
+  LAUNCH_CHECK(h);
+  return 0;
+}
+
+// kg == nullptr: arg-max of the first pick only.  partials: acq_partials_doubles(); best: [value, index bits]
+int acq_update_launch(mfgp_ctx* h, const double* kg, double* R, long long C, int i, const double* rp, double rho,
+                      double* v, double noise_add, double* partials, double* best) {
+  int nb = (int)((C + 255) / 256);
+  if (nb > RED_BLOCKS) nb = RED_BLOCKS;
+  if (nb < 1) nb = 1;
+  long long* pidx = reinterpret_cast<long long*>(partials + RED_BLOCKS);
+  prof_begin(h, PC_ARGMAX);
+  acq_update_kernel<<<nb, 256, 0, h->stream>>>(kg, R, C, i, rp, rho, v, noise_add, partials, pidx);
+  prof_end(h, PC_ARGMAX);
+  LAUNCH_CHECK(h);
+  argmax_stage2_kernel<<<1, 256, 0, h->stream>>>(partials, pidx, nb, best, reinterpret_cast<long long*>(best + 1));
+  LAUNCH_CHECK(h);
+  return 0;
+}
+
+int acq_gather_launch(mfgp_ctx* h, const double* best, const double* v, const double* cands, int D,
+                      const double* R, long long C, int nr, int q, double* out) {
+  acq_gather_kernel<<<1, 128, 0, h->stream>>>(best, reinterpret_cast<const long long*>(best + 1), v, cands, D, R, C,
+                                               nr, q, out);
   LAUNCH_CHECK(h);
   return 0;
 }

@@ -1,9 +1,10 @@
 """Multi-GPU plumbing (SURVEY.md section 8e): one process per GPU, torch.distributed.
 
 Only the naturally sharded work is partitioned -- test points x MC samples and acquisition
-candidates -- by contiguous ranges with no data-path collective.  NCCL is used for exactly two
-things: broadcasting the factorised training state after a fit, and gathering one
-(value, global index) pair per rank for the arg-max.  The same code runs on gloo for CPU tests.
+candidates -- by contiguous ranges with no data-path collective.  NCCL is used for broadcasting the
+factorised training state after a fit, gathering one (value, global index) pair per rank for the
+arg-max, and (batch acquisition) broadcasting the winner's small pivot record from the rank that owns
+it.  The same code runs on gloo for CPU tests.
 """
 import numpy as np
 import torch
@@ -58,6 +59,26 @@ def gather_argmax(local_val, local_idx, device=None):
     tdist.all_gather(vs, v)
     tdist.all_gather(is_, i)
     return combine_argmax([t.item() for t in vs], [t.item() for t in is_])
+
+
+def shard_owner(index, n, world):
+    """Rank whose shard_range(n, rank, world) holds the global `index`."""
+    base, extra = divmod(int(n), int(world))
+    index = int(index)
+    if index < extra * (base + 1):
+        return index // (base + 1)
+    return extra + (index - extra * (base + 1)) // base
+
+
+def broadcast_record(rec, src, device=None):
+    """The f64 vector `rec` of rank `src` on every rank, bit for bit (the batch acquisition's pivot record: every rank
+    conditions its shard on the global winner).  Every rank passes a vector of the same length."""
+    rec = np.ascontiguousarray(rec, dtype=np.float64)
+    if not is_dist():
+        return rec.copy()
+    t = torch.from_numpy(rec.copy()).to(coll_device(device))
+    tdist.broadcast(t, src=int(src))
+    return t.cpu().numpy()
 
 
 def restart_share(num_restarts, rank, world):
