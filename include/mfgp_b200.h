@@ -150,6 +150,22 @@ size_t mfgp_predict_ws_bytes(int N, long long cols);
 int mfgp_predict(mfgp_handle_t h, const mfgp_level_t* gp, const double* d_Xnew, long long M,
                  double* d_mean, double* d_var, int include_noise, double* d_ws, size_t ws_bytes);
 
+/* K6d -- predictive gradients.  Replaces GPy's GP.predictive_gradients [GPy-recall]: for the query rows q_c of d_Xnew
+ * (M, D), dmean[c][j] = d mu(q_c) / d q_j = sum_k alpha_k dk(q_c, X_k)/dq_j and dvar[c][j] = d var / d q_j =
+ * -2 sum_k u_kc dk(q_c, X_k)/dq_j with u_c = K_y^-1 k_c (k(q, q) is constant for both kernels).  dvar is the
+ * derivative of the UNCLIPPED latent variance; the noise is a constant.  Both (M, D) row-major.
+ * By-products (optional, NULL to skip): d_mean and d_var are mfgp_predict's outputs (var clipped at 1e-15, plus the
+ * noise if include_noise), equal to them to round-off (other summation orders), so that an optimiser gets f and g
+ * from one call.  d_dvar == NULL: mean-only mode -- no W, no scratch (d_ws may be NULL), d_var must be NULL.
+ * Otherwise d_ws holds W^T and the per-chunk blocks: at least mfgp_predictive_gradients_ws_bytes(N, 128); chunks
+ * are sized from ws_bytes.  A query's outputs do not depend on the chunk size or on the other queries of the call.
+ * Asynchronous on the handle's stream, like mfgp_predict. */
+size_t mfgp_predictive_gradients_ws_bytes(int N, long long cols);
+int mfgp_predictive_gradients(mfgp_handle_t h, const mfgp_level_t* gp, const double* d_Xnew, long long M,
+                              double* d_dmean /* (M, D) */, double* d_dvar /* (M, D) or NULL */,
+                              double* d_mean /* (M) or NULL */, double* d_var /* (M) or NULL */,
+                              int include_noise, double* d_ws, size_t ws_bytes);
+
 /* K6, latency path: M <= mfgp_predict_small_max_rows() query rows given in HOST memory, results to HOST memory,
  * one or two launches and ONE synchronisation (query rows and results travel through pinned host memory
  * mapped into the device).  This is what a single objective evaluation of the reference's default acquisition

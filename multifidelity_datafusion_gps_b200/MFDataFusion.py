@@ -224,6 +224,63 @@ class MultifidelityDataFusion(AbstractMFGP):
         self._apply_add_noise()
         return self.hf_model.predict_device(dXa, True, True)
 
+    # -- predictive gradients (extension) -----------------------------------------------------------
+    def _f_low_jacobian(self, locations):
+        """d f_low / d x at (n, d) host locations -> (n, d).  A data-driven LF level: its mean-only predictive
+        gradients on the device.  A callable: its ``gradient(locations)`` if it has one, otherwise central differences
+        (step 1e-6 max(1, |x_i|)) over the 2 d shifted location sets in one vectorised f_low evaluation."""
+        n, d = locations.shape
+        if self.data_driven_lf_approach:
+            dmean, _, _, _ = self.lf_model.predictive_gradients_device(gp.to_device(locations, self.device), False)
+            return dmean.cpu().numpy()
+        grad = getattr(self.f_low, "gradient", None)
+        if grad is not None:
+            J = np.asarray(grad(locations), dtype=np.float64)
+            assert J.shape == (n, d), "f_low.gradient must return one row of d partial derivatives per location"
+            return J
+        step = 1e-6 * np.maximum(1.0, np.abs(locations))                       # (n, d)
+        shifted = np.empty((2, d, n, d))
+        for i in range(d):
+            for s, sign in enumerate((1.0, -1.0)):
+                shifted[s, i] = locations
+                shifted[s, i, :, i] += sign * step[:, i]
+        vals = self._f_low_batched(shifted.reshape(2 * d * n, 1, d)).reshape(2, d, n)
+        return ((vals[0] - vals[1]) / (2.0 * step.T)).T
+
+    def predictive_gradients_device(self, dX, include_noise=True):
+        """dX (M, d) CUDA -> (dmean (M, d), dvar (M, d), mean (M,), var (M,)) CUDA tensors: the gradients of the
+        predictive mean and of the latent variance with respect to the plain inputs x, by the chain rule through the
+        augmentation [x, f_low(x + o_e tau)]; mean and var are ``predict``'s outputs to round-off."""
+        d, E = self.input_dim, self.augm_iterator.new_entries_count()
+        self._apply_add_noise()
+        dXa = self._augment_device(dX)
+        gm, gv, mean, var = self.hf_model.predictive_gradients_device(dXa, True, include_noise)
+        offs = torch.from_numpy(np.ascontiguousarray(self.augm_iterator.offset_table() * self.tau)).to(dX.device)
+        loc = (dX[:, None, :] + offs[None, :, :]).reshape(-1, d)
+        J = torch.from_numpy(np.ascontiguousarray(self._f_low_jacobian(loc.cpu().numpy()))).to(dX.device)
+        J = J.reshape(-1, E, d)
+        dmean, dvar = gm[:, :d].clone(), gv[:, :d].clone()
+        for e in range(E):              # element-wise, in a fixed order: a row's result does not depend on M
+            dmean += gm[:, d + e, None] * J[:, e, :]
+            dvar += gv[:, d + e, None] * J[:, e, :]
+        return dmean, dvar, mean, var
+
+    def predictive_gradients(self, X):
+        """GP.predictive_gradients with respect to the plain inputs: (dmu_dX (M, d, 1), dv_dX (M, d)) as NumPy."""
+        X = np.ascontiguousarray(X, dtype=np.float64)
+        assert X.ndim == 2 and X.shape[1] == self.input_dim
+        dmean, dvar, _, _ = self.predictive_gradients_device(gp.to_device(X, self.device))
+        return dmean.cpu().numpy()[:, :, None], dvar.cpu().numpy()
+
+    def variance_and_gradient(self, X):
+        """(var (M,), dvar (M, d)) as NumPy: the predictive variance as ``predict`` reports it (to round-off) and its
+        gradient, which is zero where the clip at 1e-15 holds the latent variance.  What LBFGSBMaximizer asks."""
+        X = np.ascontiguousarray(X, dtype=np.float64)
+        _, dvar, _, var = self.predictive_gradients_device(gp.to_device(X, self.device), include_noise=False)
+        v, g = var.cpu().numpy(), dvar.cpu().numpy()
+        g[v <= 1e-15] = 0.0
+        return v + self.hf_model.likelihood.variance, g
+
     def get_mse(self, X_test, Y_test):
         assert len(X_test) == len(Y_test), 'unequal number of X and y values'
         assert X_test.shape[1] == self.input_dim, 'wrong input value dimension'

@@ -25,6 +25,7 @@ EXPORTS = [
     "mfgp_lml_grad_timed", "mfgp_lml_grad_batch_max", "mfgp_lml_grad_batch", "mfgp_append_point", "mfgp_potrf", "mfgp_trtri", "mfgp_lauum", "mfgp_predict_ws_bytes",
     "mfgp_predict", "mfgp_predict_small_max_rows", "mfgp_predict_small", "mfgp_point_service_start", "mfgp_point_service_eval", "mfgp_point_service_stop", "mfgp_point_service_relaunches", "mfgp_augment", "mfgp_predict_mc_ws_bytes", "mfgp_predict_mc", "mfgp_predict_mc_chain", "mfgp_predict_mc_joint_ws_bytes", "mfgp_predict_mc_joint",
     "mfgp_predict_mc_delays", "mfgp_fill_normal",
+    "mfgp_predictive_gradients_ws_bytes", "mfgp_predictive_gradients",
     "mfgp_argmax", "mfgp_acq_batch_ws_bytes", "mfgp_acq_batch_begin", "mfgp_acq_batch_step",
     "mfgp_pce_ws_bytes", "mfgp_pce_project",
 ]
@@ -112,6 +113,9 @@ def load_library():
                                            vp, c_sz]
     lib.mfgp_fill_normal.argtypes = [vp, c_ull, c_ll, c_ll, vp]
     lib.mfgp_argmax.argtypes = [vp, vp, c_ll, vp, vp]
+    lib.mfgp_predictive_gradients_ws_bytes.argtypes = [c_int, c_ll]
+    lib.mfgp_predictive_gradients_ws_bytes.restype = c_sz
+    lib.mfgp_predictive_gradients.argtypes = [vp, ctypes.POINTER(Level), vp, c_ll, vp, vp, vp, vp, c_int, vp, c_sz]
     lib.mfgp_acq_batch_ws_bytes.argtypes = [c_int, c_ll, c_int]
     lib.mfgp_acq_batch_ws_bytes.restype = c_sz
     lib.mfgp_acq_batch_begin.argtypes = [vp, ctypes.POINTER(Level), vp, c_ll, c_int, c_int, vp, c_sz, vp, vp, vp]
@@ -124,7 +128,7 @@ def load_library():
         fn = getattr(lib, name)
         if name not in ("mfgp_last_error", "mfgp_launch_count", "mfgp_predict_ws_bytes", "mfgp_pce_ws_bytes",
                         "mfgp_predict_mc_joint_ws_bytes", "mfgp_predict_mc_ws_bytes", "mfgp_point_service_relaunches",
-                        "mfgp_acq_batch_ws_bytes"):
+                        "mfgp_acq_batch_ws_bytes", "mfgp_predictive_gradients_ws_bytes"):
             fn.restype = c_int
     _lib = lib
     return lib

@@ -2,6 +2,7 @@
 (reference: src/adaptation_maximizers/; ``CandidateSetMaximizer`` is the GPU candidate-set arg-max)."""
 from .abstract_maximizer import AbstractMaximizer
 from .candidate_set_maximizer import CandidateSetMaximizer
+from .lbfgsb_maximizer import LBFGSBMaximizer
 from .scipydirect_wrapper import ScipyDirectMaximizer
 
-__all__ = ["AbstractMaximizer", "CandidateSetMaximizer", "ScipyDirectMaximizer"]
+__all__ = ["AbstractMaximizer", "CandidateSetMaximizer", "LBFGSBMaximizer", "ScipyDirectMaximizer"]

@@ -536,6 +536,159 @@ constexpr size_t cross_smem(int D) {
   return fm::EXP_TBL_BYTES + ((size_t)D * BT + 2 * (size_t)(D + 1) * BT) * sizeof(double);
 }
 
+// ---- K6d: predictive gradients of one level -------------------------------------------------------------------
+//   dmean[c][j] = 2 sum_k alpha_k (q_cj - X_kj) w_kj,   dvar[c][j] = -4 sum_k u_kc (q_cj - X_kj) w_kj
+//   w = ax k12 + a3 k3 for an x column, az k12 for a z column (u_c = K_y^-1 k_c, rows of Ut = Ks K_y^-1);
+// by-products mean[c] = sum_k alpha_k k and quad[c] = sum_k u_kc k (the variance is kdiag - quad).
+// A CTA owns 128 queries and walks the training points in double-buffered stages of GK (cp.async: their rows,
+// alpha, and the matching 128 x GK block of Ut, whose rows are contiguous in global memory).  Thread t serves
+// query t/2 and the stage's points k = 2m + t%2; the two partial sums of a query meet in one shuffle at the end, so
+// every sum runs in a fixed order that depends on nothing but N.  DT = 0 (runtime width) accumulates the gradient
+// columns [j0, j0 + GJ) per launch.
+constexpr int GK = 16;           // training points per stage
+constexpr int GU_LD = GK + 2;    // Ut stage row stride: a half-warp's reads (8 queries x 2 points) hit 16 bank pairs
+constexpr int GJ = 8;            // gradient columns per launch of the runtime-width kernel
+
+template <int DT, int E>
+__global__ void __launch_bounds__(256, 2)
+    cross_grad_kernel(KParams kp, const double* __restrict__ X, int N, const double* __restrict__ alpha,
+                      const double* __restrict__ Ut, long ldu, const double* __restrict__ Xq, long ncols, int j0,
+                      double* __restrict__ dmean, double* __restrict__ dvar, double* __restrict__ mean,
+                      double* __restrict__ quad) {
+  extern __shared__ __align__(16) double dsm[];   // exp table | sXq[D][BT] | 2 x (sXk[D][GK] | alpha[GK] | sU[BT][GU_LD])
+  const int D = DT > 0 ? DT : kp.D, d = DT > 0 ? DT - E : kp.d;
+  constexpr int NJ = DT > 0 ? DT : GJ;
+  double* sXq = dsm + fm::EXP_TBL_DOUBLES;
+  double* sSt = sXq + D * BT;
+  const int stage = D * GK + GK + BT * GU_LD;
+  fm::load_exp_table(dsm, kp.exp_tbl);
+  const KEval<DT, E> ke(kp, fm::lane_table(dsm));
+  const bool has3 = ke.has3, want_u = Ut != nullptr;
+  const double ax = kp.ax, az = kp.az, a3 = kp.a3;
+  const long c0 = (long)blockIdx.x * BT;
+  const int cl = threadIdx.x >> 1, h = threadIdx.x & 1;
+  {
+    const long left = ncols - c0;
+    prefetch_rows<DT>(sXq, Xq + c0 * D, left > BT ? BT : (int)left, D, 0);
+  }
+  auto prefetch = [&](int s, int buf) {
+    double* p = sSt + buf * stage;
+    const int k0 = s * GK;
+    for (int i = threadIdx.x; i < GK * D; i += blockDim.x) {   // rows k0.. are one contiguous run of X
+      const int r = i / D, dd = i - r * D;
+      const bool ok = k0 + r < N;
+      cp_async8_zfill(p + dd * GK + r, ok ? X + (long)k0 * D + i : X, ok);
+    }
+    if (threadIdx.x < GK) {
+      const bool ok = k0 + (int)threadIdx.x < N;
+      cp_async8_zfill(p + D * GK + threadIdx.x, ok ? alpha + k0 + threadIdx.x : alpha, ok);
+    }
+    if (want_u) {
+      double* su = p + D * GK + GK;
+      for (int i = threadIdx.x; i < BT * GK; i += blockDim.x) {
+        const int r = i / GK, kk = i - r * GK;
+        const bool ok = c0 + r < ncols && k0 + kk < N;
+        cp_async8_zfill(su + r * GU_LD + kk, ok ? Ut + (c0 + r) * ldu + k0 + kk : Ut, ok);
+      }
+    }
+  };
+  const int nst = (N + GK - 1) / GK;
+  prefetch(0, 0);
+  cp_async_commit();
+  double gm[NJ], gv[NJ], q[DT > 0 ? DT : 1];
+#pragma unroll
+  for (int j = 0; j < NJ; j++) gm[j] = gv[j] = 0.0;
+  double am = 0.0, aq = 0.0;
+  int buf = 0;
+  for (int s = 0; s < nst; s++, buf ^= 1) {
+    if (s + 1 < nst) prefetch(s + 1, buf ^ 1);
+    cp_async_commit();
+    cp_async_wait<1>();
+    __syncthreads();
+    if (DT > 0 && s == 0) {
+#pragma unroll
+      for (int dd = 0; dd < (DT > 0 ? DT : 1); dd++) q[dd] = sXq[dd * BT + cl];
+    }
+    const double* sXk = sSt + buf * stage;
+    const double* sA = sXk + D * GK;
+    const double* sU = sA + GK;
+#pragma unroll 2
+    for (int m = 0; m < GK / 2; m++) {
+      const int k = 2 * m + h;
+      double t[NJ];
+      double rx = 0.0, rz = 0.0;
+      if (DT > 0) {
+#pragma unroll
+        for (int dd = 0; dd < NJ; dd++) {
+          t[dd] = q[dd] - sXk[dd * GK + k];
+          if (dd < DT - E) rx = fma(t[dd], t[dd], rx);
+          else rz = fma(t[dd], t[dd], rz);
+        }
+      } else {
+        for (int dd = 0; dd < D; dd++) {
+          const double tt = sXq[dd * BT + cl] - sXk[dd * GK + k];
+          if (dd < d) rx = fma(tt, tt, rx);
+          else rz = fma(tt, tt, rz);
+        }
+#pragma unroll
+        for (int jj = 0; jj < NJ; jj++) {
+          const int j = j0 + jj;
+          t[jj] = j < D ? sXq[j * BT + cl] - sXk[j * GK + k] : 0.0;
+        }
+      }
+      const double k12 = ke.k12(rx, rz);
+      const double k3 = has3 ? ke.k3(rx) : 0.0;
+      const double kv = k12 + k3;
+      const double gx = has3 ? fma(ax, k12, a3 * k3) : ax * k12, gz = az * k12;
+      const double a = sA[k];
+      am = fma(a, kv, am);
+      const double wax = a * gx, waz = a * gz;
+#pragma unroll
+      for (int jj = 0; jj < NJ; jj++) {
+        const bool xcol = DT > 0 ? jj < DT - E : j0 + jj < d;
+        gm[jj] = fma(t[jj], xcol ? wax : waz, gm[jj]);
+      }
+      if (want_u) {
+        const double u = sU[cl * GU_LD + k];
+        aq = fma(u, kv, aq);
+        const double wux = u * gx, wuz = u * gz;
+#pragma unroll
+        for (int jj = 0; jj < NJ; jj++) {
+          const bool xcol = DT > 0 ? jj < DT - E : j0 + jj < d;
+          gv[jj] = fma(t[jj], xcol ? wux : wuz, gv[jj]);
+        }
+      }
+    }
+    __syncthreads();   // all readers done with this buffer before the next iteration refills it
+  }
+  cp_async_wait<0>();
+  // the two halves of a query sit in adjacent lanes: one shuffle, the same sum in both
+#pragma unroll
+  for (int jj = 0; jj < NJ; jj++) {
+    gm[jj] += __shfl_xor_sync(0xffffffffu, gm[jj], 1);
+    gv[jj] += __shfl_xor_sync(0xffffffffu, gv[jj], 1);
+  }
+  am += __shfl_xor_sync(0xffffffffu, am, 1);
+  aq += __shfl_xor_sync(0xffffffffu, aq, 1);
+  const long c = c0 + cl;
+  if (h != 0 || c >= ncols) return;
+#pragma unroll
+  for (int jj = 0; jj < NJ; jj++) {
+    const int j = (DT > 0 ? 0 : j0) + jj;
+    if (DT == 0 && j >= D) break;
+    dmean[c * D + j] = 2.0 * gm[jj];
+    if (dvar) dvar[c * D + j] = -4.0 * gv[jj];
+  }
+  if (DT > 0 || j0 == 0) {
+    if (mean) mean[c] = am;
+    if (quad) quad[c] = aq;
+  }
+}
+
+constexpr size_t xgrad_smem(int D) {
+  return fm::EXP_TBL_BYTES + ((size_t)D * BT + 2 * ((size_t)D * GK + GK + (size_t)BT * GU_LD)) * sizeof(double);
+}
+
 constexpr size_t asm_smem(int D) { return fm::EXP_TBL_BYTES + (size_t)2 * 2 * D * BT * sizeof(double); }
 constexpr size_t grad_smem(int D) { return fm::EXP_TBL_BYTES + (size_t)2 * 2 * (D + 1) * BT * sizeof(double); }
 
@@ -551,13 +704,17 @@ int assemble_configure(mfgp_ctx* h) {
   CUDA_TRY(h, cudaFuncSetAttribute(assemble_kernel<true, 0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
   CUDA_TRY(h, cudaFuncSetAttribute(assemble_kernel<false, 0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
   CUDA_TRY(h, cudaFuncSetAttribute(grad_reduce_kernel<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, gmax));
+  CUDA_TRY(h, cudaFuncSetAttribute(cross_grad_kernel<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                   (int)xgrad_smem(MFGP_MAX_D)));
 #define MFGP_CFG(DT, E)                                                                                   \
   CUDA_TRY(h, cudaFuncSetAttribute(assemble_kernel<true, DT, E>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
                                    (int)asm_smem(DT)));                                                   \
   CUDA_TRY(h, cudaFuncSetAttribute(grad_reduce_kernel<DT, E>, cudaFuncAttributeMaxDynamicSharedMemorySize,    \
                                    (int)grad_smem(DT)));                                                  \
   CUDA_TRY(h, cudaFuncSetAttribute(cross_tile_kernel<DT, E>, cudaFuncAttributeMaxDynamicSharedMemorySize,     \
-                                   (int)cross_smem(DT)));
+                                   (int)cross_smem(DT)));                                                 \
+  CUDA_TRY(h, cudaFuncSetAttribute(cross_grad_kernel<DT, E>, cudaFuncAttributeMaxDynamicSharedMemorySize,     \
+                                   (int)xgrad_smem(DT)));
   MFGP_SHAPES(MFGP_CFG)
 #undef MFGP_CFG
   return 0;
@@ -644,4 +801,32 @@ int cross_tile_launch(mfgp_ctx* h, const KParams& kp, const double* X, int N, in
   MFGP_SHAPES(MFGP_RUN)
 #undef MFGP_RUN
   return done ? 1 : 0;
+}
+
+// K6d launcher: gradients of the queries Xq[0, ncols) (see cross_grad_kernel).  Ut == nullptr: mean mode (dvar and
+// quad are not written).  Specialised shapes take one launch; the runtime-width kernel one per GJ gradient columns.
+int cross_grad_launch(mfgp_ctx* h, const KParams& kp, const double* X, int N, const double* alpha, const double* Ut,
+                      long long ldu, const double* Xq, long long ncols, double* dmean, double* dvar, double* mean,
+                      double* quad) {
+  if (ncols <= 0) return 0;
+  const Shape sh = shape_of(kp);
+  const unsigned grid = (unsigned)((ncols + BT - 1) / BT);
+  const size_t smem = xgrad_smem(kp.D);
+  prof_begin(h, PC_CROSSGEN);
+  bool done = false;
+#define MFGP_RUN(DT_, E_)                                                                                     \
+  if (!done && sh.DT == DT_ && sh.E == E_) {                                                                  \
+    cross_grad_kernel<DT_, E_><<<grid, 256, smem, h->stream>>>(kp, X, N, alpha, Ut, (long)ldu, Xq, (long)ncols, 0, \
+                                                               dmean, dvar, mean, quad);                      \
+    done = true;                                                                                              \
+  }
+  MFGP_SHAPES(MFGP_RUN)
+#undef MFGP_RUN
+  if (!done)
+    for (int j0 = 0; j0 < kp.D; j0 += GJ)
+      cross_grad_kernel<0, 0><<<grid, 256, smem, h->stream>>>(kp, X, N, alpha, Ut, (long)ldu, Xq, (long)ncols, j0,
+                                                              dmean, dvar, mean, quad);
+  prof_end(h, PC_CROSSGEN);
+  LAUNCH_CHECK(h);
+  return 0;
 }

@@ -590,6 +590,56 @@ int mfgp_predict(mfgp_handle_t h, const mfgp_level_t* gp, const double* d_Xnew, 
   return predict_impl(h, gp, kp, d_Xnew, M, d_mean, d_var, include_noise, d_ws, ws_bytes);
 }
 
+// ---- K6d predictive gradients (math: assemble.cu, cross_grad_kernel) -------------------------------------------
+// Scratch: W^T (npad^2) | per chunk Ks, reused for Ut = Ks K_y^-1 (chunk x npad) | Tt (chunk x npad).
+size_t mfgp_predictive_gradients_ws_bytes(int N, long long cols) {
+  const long long npad = mfgp_padded_n(N);
+  const long long cp = ((cols < 1 ? 1 : cols) + 127) / 128 * 128;
+  return (size_t)(npad * npad + 2 * npad * cp) * sizeof(double);
+}
+
+int mfgp_predictive_gradients(mfgp_handle_t h, const mfgp_level_t* gp, const double* d_Xnew, long long M,
+                              double* d_dmean, double* d_dvar, double* d_mean, double* d_var, int include_noise,
+                              double* d_ws, size_t ws_bytes) {
+  ENTER(h);
+  KParams kp;
+  int rc = level_kparams(h, gp, &kp);
+  if (rc) return rc;
+  ARG_CHECK(h, M >= 0 && (d_Xnew != nullptr || M == 0) && d_dmean != nullptr);
+  ARG_CHECK(h, d_dvar != nullptr || d_var == nullptr);   // the variance needs W, as its gradient does
+  const int N = gp->N, D = gp->D, npad = mfgp_padded_n(N);
+  long long chunk = M;
+  double *Wt = nullptr, *Ks = nullptr, *Tt = nullptr;
+  if (d_dvar) {
+    ARG_CHECK(h, gp->d_W != nullptr && d_ws != nullptr);
+    ARG_CHECK(h, ws_bytes >= mfgp_predictive_gradients_ws_bytes(N, 128));
+    const long long avail = (long long)(ws_bytes / sizeof(double)) - (long long)npad * npad;
+    chunk = whole_waves(avail / (2LL * npad) / 128 * 128);
+    Wt = d_ws;
+    Ks = Wt + (long long)npad * npad;
+    Tt = Ks + chunk * npad;
+  }
+  if (M == 0) return 0;
+  if (d_dvar && (rc = transpose_launch(h, gp->d_W, npad, Wt))) return rc;
+  for (long long c0 = 0; c0 < M; c0 += chunk) {
+    const long long ncols = (M - c0 < chunk) ? (M - c0) : chunk;
+    const long long cols_pad = (ncols + 127) / 128 * 128;
+    const double* Xq = d_Xnew + c0 * D;
+    if (d_dvar) {
+      if ((rc = cross_gen_launch(h, kp, gp->d_X, N, npad, gp->d_alpha, Xq, ncols, cols_pad, Ks, nullptr))) return rc;
+      if ((rc = kinv_rows(h, gp->d_W, Wt, npad, Ks, cols_pad, Tt, Ks))) return rc;
+    }
+    if ((rc = cross_grad_launch(h, kp, gp->d_X, N, gp->d_alpha, d_dvar ? Ks : nullptr, npad, Xq, ncols,
+                                d_dmean + c0 * D, d_dvar ? d_dvar + c0 * D : nullptr, d_mean ? d_mean + c0 : nullptr,
+                                d_var ? d_var + c0 : nullptr)))
+      return rc;
+    if (d_var && (rc = finish_var_launch(h, d_var + c0, ncols, kp.kdiag, include_noise ? kp.noise : 0.0, d_var + c0,
+                                         false)))
+      return rc;
+  }
+  return 0;
+}
+
 int mfgp_predict_small_max_rows(void) { return 16; }
 
 int mfgp_predict_small(mfgp_handle_t h, const mfgp_level_t* hf, const mfgp_level_t* lf, const double* h_X,

@@ -170,6 +170,10 @@ int small_batch_max();
 int small_lml_batch_launch(mfgp_ctx* h, const KParams* kps, const double* diag_add, int B, const double* X,
                            const double* y, int N, double* d_out, int* d_info, int want_grad);
 int trmm_store(mfgp_ctx* h, const double* W, int npad, const double* Ks, long long cols_pad, double* T);
+// Ut = Ks K_y^-1 for the rows of Ks (cols_pad x npad, like Ut and the scratch Tt), Wt = W^T (npad x npad)
+int kinv_rows(mfgp_ctx* h, const double* W, const double* Wt, int npad, const double* Ks, long long cols_pad,
+              double* Tt, double* Ut);
+int transpose_launch(mfgp_ctx* h, const double* A, int n, double* At);   // At = A^T, n x n, n multiple of 32
 // C(lower, n x n, ld = n) -= T^T T for T (k x n, ld = ldt); n, k multiples of 128
 int syrk_tn_sub(mfgp_ctx* h, const double* T, long long ldt, int k, double* C, int n);
 // Z[i][c] = sum_{k<=i} L[i][k] E[k][c]   (L: n x n lower with explicit zeros above the diagonal inside its
@@ -182,5 +186,8 @@ int assemble_launch(mfgp_ctx* h, const KParams& kp, const double* X, int N, doub
                     double* K, long long ldk, int uplo, int npad_identity);
 int cross_tile_launch(mfgp_ctx* h, const KParams& kp, const double* X, int N, int npad, const double* alpha,
                       const double* Xq, long long ncols, long long cols_pad, double* Ks, double* mean);
+int cross_grad_launch(mfgp_ctx* h, const KParams& kp, const double* X, int N, const double* alpha, const double* Ut,
+                      long long ldu, const double* Xq, long long ncols, double* dmean, double* dvar, double* mean,
+                      double* quad);
 int grad_reduce_launch(mfgp_ctx* h, const KParams& kp, const double* X, int N, const double* Kinv,
                        long long ld, const double* alpha, double* d_out8);

@@ -158,6 +158,7 @@ struct GemmParams {
   double alpha, beta;
   int lower_only;                      // enumerate only tiles with ti >= tj (M == N)
   int kb_row, kb_col, ke_row;          // triangular operands: k >= row0 / k >= col0 / k < row0+BM
+  int ke_col;                          //                      k < col0+BN
   // batch of equally shaped, independent products along a diagonal (the nodes of one level of the
   // triangular-inverse recursion): node b works on A + b*stride, B + b*stride, C + b*stride
   int batch;                           // number of nodes (0 or 1: plain product)
@@ -194,6 +195,7 @@ __global__ void __launch_bounds__(T::THREADS) gemm_kernel(GemmParams p) {
   if (p.kb_row) kb = max(kb, row0);
   if (p.kb_col) kb = max(kb, col0);
   if (p.ke_row) ke = min(ke, row0 + T::BM);
+  if (p.ke_col) ke = min(ke, col0 + T::BN);
 
   double acc[T::MT][T::NT][2];
 #pragma unroll
@@ -587,7 +589,7 @@ struct GemmTmaParams {
   int M, N, K;
   double alpha, beta;
   int lower_only;
-  int kb_row, kb_col, ke_row;
+  int kb_row, kb_col, ke_row, ke_col;
   int batch;
   long c_batch_stride;     // elements between the C blocks of consecutive nodes
   int a_batch_rows, a_batch_k, b_batch_rows, b_batch_k;   // coordinate shifts per node
@@ -634,6 +636,7 @@ __global__ void __launch_bounds__(T::THREADS, 1)
   if (p.kb_row) kb = max(kb, row0);
   if (p.kb_col) kb = max(kb, col0);
   if (p.ke_row) ke = min(ke, row0 + T::BM);
+  if (p.ke_col) ke = min(ke, col0 + T::BN);
   const int nk = ke > kb ? (ke - kb) / BK : 0;
   if (tid == 0) {
     for (int s = 0; s < tma::NST; s++) {
@@ -780,6 +783,7 @@ __global__ void __launch_bounds__(T::THREADS, 1)
   if (p.kb_row) kb = max(kb, row0);
   if (p.kb_col) kb = max(kb, col0);
   if (p.ke_row) ke = min(ke, row0 + T::BM);
+  if (p.ke_col) ke = min(ke, col0 + T::BN);
   const int nk = ke > kb ? (ke - kb) / BK : 0;
   if (tid == 0) {
     for (int s = 0; s < tma::NST; s++) {

@@ -634,7 +634,7 @@ static int try_gemm_tma(mfgp_ctx* h, const dg::GemmParams& p, int cls) {
   dg::GemmTmaParams q;
   memset(&q, 0, sizeof(q));
   q.C = p.C; q.ldc = p.ldc; q.M = p.M; q.N = p.N; q.K = p.K; q.alpha = p.alpha; q.beta = p.beta;
-  q.lower_only = p.lower_only; q.kb_row = p.kb_row; q.kb_col = p.kb_col; q.ke_row = p.ke_row;
+  q.lower_only = p.lower_only; q.kb_row = p.kb_row; q.kb_col = p.kb_col; q.ke_row = p.ke_row; q.ke_col = p.ke_col;
   q.batch = p.batch; q.c_batch_stride = c_stride;
   q.a_batch_rows = (int)a_rows_shift; q.a_batch_k = (int)a_k_shift;
   q.b_batch_rows = (int)b_rows_shift; q.b_batch_k = (int)b_k_shift;
@@ -683,7 +683,7 @@ static int try_gemm_tma_mc(mfgp_ctx* h, const dg::GemmParams& p, int cls) {
   dg::GemmTmaParams q;
   memset(&q, 0, sizeof(q));
   q.C = p.C; q.ldc = p.ldc; q.M = p.M; q.N = p.N; q.K = p.K; q.alpha = p.alpha; q.beta = p.beta;
-  q.lower_only = p.lower_only; q.kb_row = p.kb_row; q.kb_col = p.kb_col; q.ke_row = p.ke_row;
+  q.lower_only = p.lower_only; q.kb_row = p.kb_row; q.kb_col = p.kb_col; q.ke_row = p.ke_row; q.ke_col = p.ke_col;
   q.batch = p.batch; q.c_batch_stride = c_stride;
   q.a_batch_rows = q.a_batch_k = q.b_batch_rows = q.b_batch_k = (int)n_shift;
   prof_begin(h, cls);
@@ -1076,6 +1076,40 @@ int trmm_store(mfgp_ctx* h, const double* W, int npad, const double* Ks, long lo
   dg::GemmParams p = gp(W, npad, Ks, npad, T, cols_pad, npad, (int)cols_pad, npad, 1.0, 0.0);
   p.ke_row = 1;
   return launch_gemm<true, true>(h, p, PC_MISC);
+}
+
+// Both products are NT (k-contiguous operands): the cp.async and TMA kernels that launch_gemm picks between share
+// one accumulation order, so a row's result does not depend on how many rows share the call.  (U = W^T T as a TT
+// product would go through gemm_tma_mc_kernel from one wave of tiles on, whose k order differs.)
+//   Tt[c][i] = sum_{k<=i} Ks[c][k] W[i][k],   Ut[c][k] = sum_{i>=k} Tt[c][i] Wt[k][i]
+int kinv_rows(mfgp_ctx* h, const double* W, const double* Wt, int npad, const double* Ks, long long cols_pad,
+              double* Tt, double* Ut) {
+  ARG_CHECK(h, npad % LEAF == 0 && cols_pad % dg::Big16::BM == 0 && cols_pad < (1LL << 31));
+  if (cols_pad == 0) return 0;
+  dg::GemmParams p = gp(Ks, npad, W, npad, Tt, npad, (int)cols_pad, npad, npad, 1.0, 0.0);
+  p.ke_col = 1;
+  int rc = launch_gemm<true, true>(h, p, PC_MISC);
+  if (rc) return rc;
+  p = gp(Tt, npad, Wt, npad, Ut, npad, (int)cols_pad, npad, npad, 1.0, 0.0);
+  p.kb_col = 1;
+  return launch_gemm<true, true>(h, p, PC_MISC);
+}
+
+__global__ void transpose_kernel(const double* __restrict__ A, int n, double* __restrict__ At) {
+  __shared__ double t[32][33];
+  const long bx = (long)blockIdx.x * 32, by = (long)blockIdx.y * 32;
+  for (int r = threadIdx.y; r < 32; r += 8) t[r][threadIdx.x] = A[(by + r) * n + bx + threadIdx.x];
+  __syncthreads();
+  for (int r = threadIdx.y; r < 32; r += 8) At[(bx + r) * n + by + threadIdx.x] = t[threadIdx.x][r];
+}
+
+int transpose_launch(mfgp_ctx* h, const double* A, int n, double* At) {
+  ARG_CHECK(h, n % 32 == 0);
+  prof_begin(h, PC_MISC);
+  transpose_kernel<<<dim3(n / 32, n / 32), dim3(32, 8), 0, h->stream>>>(A, n, At);
+  prof_end(h, PC_MISC);
+  LAUNCH_CHECK(h);
+  return 0;
 }
 
 int syrk_tn_sub(mfgp_ctx* h, const double* T, long long ldt, int k, double* C, int n) {

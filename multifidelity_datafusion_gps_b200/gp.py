@@ -618,6 +618,38 @@ class GPRegression:
                                    ws_ptr, nbytes))
         return mean, var
 
+    def predictive_gradients_device(self, dX, want_var=True, include_noise=True):
+        """dX (M, D) CUDA -> (dmean (M, D), dvar (M, D) or None, mean (M,), var (M,) or None) CUDA tensors
+        (mfgp_predictive_gradients).  dvar: gradient of the unclipped latent variance; mean and var: predict_device's
+        outputs to round-off.  want_var=False is the mean-only mode (one generator pass, no W)."""
+        h = _ffi.get_handle(self.device)
+        lvl = self.level_struct()
+        M, D = int(dX.shape[0]), self.D
+        assert dX.ndim == 2 and int(dX.shape[1]) == D, "query width must equal the level's input width"
+        new = lambda *shape: torch.empty(shape, dtype=torch.float64, device=dX.device)
+        dmean, mean = new(M, D), new(M)
+        dvar = var = None
+        ws_ptr, nbytes = None, 0
+        if want_var:
+            dvar, var = new(M, D), new(M)
+            ws_bytes = max(min(h.lib.mfgp_predictive_gradients_ws_bytes(self.N, max(M, 1)), 1 << 30),
+                           h.lib.mfgp_predictive_gradients_ws_bytes(self.N, 128))
+            ws = workspace(self.device, ws_bytes)
+            ws_ptr, nbytes = ws.data_ptr(), ws.numel() * 8
+        h.check(h.lib.mfgp_predictive_gradients(h.h, ctypes.byref(lvl), dX.data_ptr(), M, dmean.data_ptr(),
+                                                dvar.data_ptr() if want_var else None, mean.data_ptr(),
+                                                var.data_ptr() if want_var else None, int(include_noise),
+                                                ws_ptr, nbytes))
+        return dmean, dvar, mean, var
+
+    def predictive_gradients(self, Xnew):
+        """GP.predictive_gradients (GPy): (dmu_dX (M, D, 1), dv_dX (M, D)) as NumPy; dv_dX is the gradient of the
+        latent variance (the noise is a constant)."""
+        Xnew = np.ascontiguousarray(Xnew, dtype=np.float64)
+        assert Xnew.ndim == 2 and Xnew.shape[1] == self.D
+        dmean, dvar, _, _ = self.predictive_gradients_device(to_device(Xnew, self.device))
+        return dmean.cpu().numpy()[:, :, None], dvar.cpu().numpy()
+
     def predict(self, Xnew, full_cov=False, include_likelihood=True):
         """GP.predict: (mean (M,1), var (M,1)) as NumPy; var includes the noise variance."""
         assert not full_cov, "full_cov is not on the reference's path"

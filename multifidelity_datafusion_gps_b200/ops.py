@@ -146,6 +146,31 @@ def predict(level, Xnew, want_var=True, include_noise=True, ws_bytes=None):
     return mean, var
 
 
+def predictive_gradients(level, Xnew, want_var=True, include_noise=True, ws_bytes=None):
+    """K6d.  Xnew (M, D) -> (dmean (M, D), dvar (M, D) or None, mean (M,), var (M,) or None); dvar is the gradient
+    of the unclipped latent variance, mean and var are predict's outputs to round-off.  want_var=False: mean-only
+    mode (no W, no scratch)."""
+    h = _ffi.get_handle(_dev(Xnew))
+    M, D = Xnew.shape
+    if D != level.struct.D:
+        raise ValueError("Xnew has %d columns, the level has D = %d" % (D, level.struct.D))
+    new = lambda *shape: torch.empty(shape, dtype=torch.float64, device=Xnew.device)
+    dmean, mean = new(M, D), new(M)
+    dvar, var, ws, nbytes = None, None, None, 0
+    if want_var:
+        dvar, var = new(M, D), new(M)
+        N = level.struct.N
+        if ws_bytes is None:
+            ws_bytes = max(min(h.lib.mfgp_predictive_gradients_ws_bytes(N, max(M, 1)), 1 << 30),
+                           h.lib.mfgp_predictive_gradients_ws_bytes(N, 128))
+        ws = new((ws_bytes + 7) // 8)
+        nbytes = ws.numel() * 8
+    ptr = lambda t: t.data_ptr() if t is not None else None
+    h.check(h.lib.mfgp_predictive_gradients(h.h, level.ref, Xnew.data_ptr(), M, dmean.data_ptr(), ptr(dvar),
+                                            mean.data_ptr(), ptr(var), int(include_noise), ptr(ws), nbytes))
+    return dmean, dvar, mean, var
+
+
 def fill_normal(seed, first, count, device):
     h = _ffi.get_handle(torch.device(device).index or 0)
     out = torch.empty(count, dtype=torch.float64, device=device)
