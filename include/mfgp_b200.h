@@ -77,8 +77,8 @@ long long mfgp_launch_count(mfgp_handle_t h);
  * event pairs on the handle's stream (first 512 launches per class).  mfgp_profile_read synchronises
  * and returns, per class, the average launch duration in ms (h_ms[10]) and the launch count
  * (h_count[10]); classes: 0 assemble, 1 potrf leaf, 2 gemm (potrf/trtri), 3 solve, 4 lauum,
- * 5 grad_reduce, 6 cross-covariance, 7 trmm+sumsq, 8 misc, 9 argmax (the batch acquisition's fused update and
- * arg-max stage). */
+ * 5 grad_reduce, 6 cross-covariance, 7 trmm+sumsq, 8 misc, 9 argmax (acquisition: the arg-max, the batch
+ * acquisition's fused update and arg-max stage, and the ALC reduction). */
 int mfgp_profile_enable(mfgp_handle_t h, int on);
 int mfgp_profile_read(mfgp_handle_t h, double* h_ms, long long* h_count);
 
@@ -298,6 +298,24 @@ int mfgp_acq_batch_begin(mfgp_handle_t h, const mfgp_level_t* gp, const double* 
 int mfgp_acq_batch_step(mfgp_handle_t h, const mfgp_level_t* gp, const double* d_cands, long long C, int q,
                         int include_noise, double jitter, int i, const double* h_rec_in, double* d_ws,
                         size_t ws_bytes, double* h_val, long long* h_idx, double* h_rec);
+
+/* K8c -- integrated-variance (ALC, "active learning Cohn") acquisition: how much acquiring candidate c lowers the
+ * weighted latent predictive variance over a reference set, at the level's current theta.  With
+ * Tt[x][i] = sum_{k<=i} k(x, X_k) W[i][k] for candidates c and references r (augmented rows, D columns):
+ *   k_n(c, r) = k(c, r) - sum_i Tt[c][i] Tt[r][i],   v_n(c) = k(c, c) - sum_i Tt[c][i]^2 (unclipped),
+ *   s^2 = noise + 1e-8 + jitter (the diagonal mfgp_append_point adds),
+ *   d_alc[c] = sum_r w_r k_n(c, r)^2 / (v_n(c) + s^2),  -inf where v_n(c) + s^2 <= 0.
+ * In exact arithmetic d_alc[c] = sum_r w_r (v_n(r) - v_{n+c}(r)) with v_{n+c} the latent variance after appending
+ * c at the same theta.  d_w (R) holds w_r >= 0, or NULL for w_r = 1/R; d_cands (C, D), d_ref (R, D), d_alc (C):
+ * DEVICE.  C >= 1, R >= 1; jitter: the level's factorisation jitter.  d_ws holds K(ref, X) and Tt_R plus per
+ * candidate chunk K(cands, X), Tt_C and G = Tt_C Tt_R^T: at least the fixed part plus one 128-column chunk
+ * (mfgp_alc_ws_bytes(N, 1, R)); chunks are sized from ws_bytes.  A candidate's value depends on nothing but the
+ * candidate, the reference set and the level: not on the chunk size or the other candidates of the call.
+ * Asynchronous on the handle's stream, like mfgp_predict; the arg-max is mfgp_argmax on d_alc.
+ * mfgp_alc_ws_bytes: the scratch for C candidates (chunk capped at 1 GiB), 0 for invalid arguments. */
+size_t mfgp_alc_ws_bytes(int N, long long C, long long R);
+int mfgp_alc(mfgp_handle_t h, const mfgp_level_t* gp, const double* d_cands, long long C, const double* d_ref,
+             long long R, const double* d_w, double jitter, double* d_alc, double* d_ws, size_t ws_bytes);
 
 /* K9 -- polynomial-chaos projection on a quadrature grid (SURVEY.md section 8f rank 2).  Replaces
  * cp.fit_quadrature / cp.E / cp.Var as src/gpc/chaospy_wrapper.py:18-29 uses them, for independent

@@ -14,6 +14,8 @@ Extensions (keyword-only, defaults reproduce the reference):
 * ``acquisition_argmax``  candidate-set arg-max of the predictive variance (used by
   ``CandidateSetMaximizer``), optionally sharded over ranks.
 * ``acquisition_batch``  greedy batch of q candidates per adaptation step (``adapt_batch_size``).
+* ``acquisition_alc``  candidate-set arg-max of the integrated-variance reduction over a reference set
+  (used by ``ALCMaximizer``), optionally sharded over ranks.
 * ``broadcast_state``  NCCL broadcast of the fitted state so that other ranks can predict.
 """
 import ctypes
@@ -25,6 +27,7 @@ import torch
 from . import _ffi, dist, gp
 from .abstractMFGP import AbstractMFGP
 from .adaptation_maximizers import AbstractMaximizer, ScipyDirectMaximizer
+from .adaptation_maximizers.alc_maximizer import alc_weights
 from .augm_iterators import BackwardAugmentation
 
 
@@ -495,7 +498,25 @@ class MultifidelityDataFusion(AbstractMFGP):
         return ("callable", id(self.f_low))
 
     def invalidate_candidate_cache(self):
+        """Drop both resident slots: the candidates' and the ALC reference rows'."""
         self._cand_cache = None
+        self._ref_cache = None
+
+    def _resident_rows(self, slot, hits, rows, lo, hi):
+        """Augmented rows of rows[lo:hi], kept on the device in the cache slot `slot` (hits counted in the attribute
+        `hits`).  The key is the array (address, shape, a checksum of a strided sample of rows), the shard and the
+        low-fidelity state."""
+        c = np.ascontiguousarray(rows, dtype=np.float64)
+        step = max(1, c.shape[0] // 4096)
+        key = (c.ctypes.data, c.shape, zlib.crc32(np.ascontiguousarray(c[::step]).tobytes()), lo, hi,
+               float(self.tau), self.augm_iterator.offset_table().tobytes(), self._lf_state_key())
+        cache = getattr(self, slot, None)
+        if cache is not None and cache[0] == key:
+            setattr(self, hits, getattr(self, hits, 0) + 1)
+            return cache[1]
+        dXa = self._augment_host_input(c[lo:hi])
+        setattr(self, slot, (key, dXa))
+        return dXa
 
     def _resident_candidates(self, candidates, lo, hi):
         """Augmented rows [c, f_low(c + o tau)] of the shard candidates[lo:hi], kept on the device.  The
@@ -504,17 +525,12 @@ class MultifidelityDataFusion(AbstractMFGP):
         first step an acquisition performs no candidate H2D / D2H and no f_low evaluation.  The cache is
         keyed on the array (address, shape, a checksum of a strided sample of rows), the shard and the
         low-fidelity state; ``invalidate_candidate_cache()`` drops it explicitly."""
-        c = np.ascontiguousarray(candidates, dtype=np.float64)
-        step = max(1, c.shape[0] // 4096)
-        key = (c.ctypes.data, c.shape, zlib.crc32(np.ascontiguousarray(c[::step]).tobytes()), lo, hi,
-               float(self.tau), self.augm_iterator.offset_table().tobytes(), self._lf_state_key())
-        cache = getattr(self, "_cand_cache", None)
-        if cache is not None and cache[0] == key:
-            self.candidate_cache_hits = getattr(self, "candidate_cache_hits", 0) + 1
-            return cache[1]
-        dXa = self._augment_host_input(c[lo:hi])
-        self._cand_cache = (key, dXa)
-        return dXa
+        return self._resident_rows("_cand_cache", "candidate_cache_hits", candidates, lo, hi)
+
+    def _resident_reference(self, reference):
+        """The ALC reference rows, augmented and resident like the candidates, in a slot of their own (hits counted
+        in ``reference_cache_hits``), so that an ALC call never evicts the candidate rows."""
+        return self._resident_rows("_ref_cache", "reference_cache_hits", reference, 0, int(reference.shape[0]))
 
     def acquisition_argmax(self, candidates, distributed=False, cache=True):
         """(index, variance) of the candidate with the largest predictive variance; lowest index on
@@ -587,6 +603,39 @@ class MultifidelityDataFusion(AbstractMFGP):
                 rec = local
             indices[i], variances[i] = idx, val
         return indices, variances
+
+    def acquisition_alc(self, candidates, reference, weights=None, distributed=False, cache=True):
+        """(index, alc) of the candidate whose acquisition most lowers the weighted mean latent predictive variance
+        over the reference rows (integrated variance, "active learning Cohn"); lowest index on ties.
+        alc(c) = sum_r w_r k_n(c, r)^2 / (v_n(c) + s^2) with k_n the latent posterior covariance, v_n(c) = k_n(c, c)
+        and s^2 = noise + 1e-8 + jitter: in exact arithmetic the drop sum_r w_r (v_n(r) - v_{n+c}(r)) that
+        ``hf_model.append_point(c)`` at the current hyper-parameters causes (mfgp_alc).  weights: (R,) >= 0, or None
+        for 1/R.  distributed / cache: as in acquisition_argmax; the reference rows are replicated on every rank and
+        stay resident in a cache slot of their own."""
+        C = int(candidates.shape[0])
+        reference = np.asarray(reference, dtype=np.float64)
+        if reference.ndim != 2 or reference.shape[1] != self.input_dim or reference.shape[0] < 1:
+            raise ValueError("reference must be a non-empty (R, %d) array" % self.input_dim)
+        w = None if weights is None else alc_weights(weights, reference.shape[0])
+        rank, world = dist.rank_world() if distributed else (0, 1)
+        lo, hi = dist.shard_range(C, rank, world)
+        val, idx = -np.inf, -1
+        if hi > lo:
+            dXa = self._resident_candidates(candidates, lo, hi) if cache else self._augment_host_input(candidates[lo:hi])
+            dXr = self._resident_reference(reference) if cache else self._augment_host_input(reference)
+            self._apply_add_noise()
+            dw = None if w is None else torch.from_numpy(w).to(dXr.device)
+            alc = self.hf_model.alc_device(dXa, dXr, dw)
+            h = _ffi.get_handle(self.device)
+            c_val, c_idx = ctypes.c_double(), ctypes.c_longlong()
+            h.check(h.lib.mfgp_argmax(h.h, alc.data_ptr(), hi - lo, ctypes.byref(c_val), ctypes.byref(c_idx)))
+            if c_val.value > -np.inf:                      # else every candidate of the shard is inadmissible
+                val, idx = c_val.value, lo + c_idx.value
+        if distributed and world > 1:
+            val, idx = dist.gather_argmax(val, idx, device="cuda:%d" % self.device)
+        if not val > -np.inf:
+            raise _ffi.MfgpError("ALC acquisition: no candidate can be appended (v_n(c) + s^2 <= 0 or NaN everywhere)")
+        return int(idx), float(val)
 
     # -- multi-GPU state ------------------------------------------------------------------------------
     def broadcast_state(self, src=0):

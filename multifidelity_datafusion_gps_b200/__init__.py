@@ -6,11 +6,12 @@ Importing the package does not touch the GPU; constructing a model does (no CPU 
 """
 from .MFDataFusion import MultifidelityDataFusion
 from .abstractMFGP import AbstractMFGP
-from .adaptation_maximizers import AbstractMaximizer, CandidateSetMaximizer, LBFGSBMaximizer, ScipyDirectMaximizer
+from .adaptation_maximizers import (AbstractMaximizer, ALCMaximizer, CandidateSetMaximizer, LBFGSBMaximizer,
+                                    ScipyDirectMaximizer)
 from .augm_iterators import AbstractAugmIterator, BackwardAugmentation, EvenAugmentation
 from .models import GPDF, GPDFC, NARGP
 from . import gpc
 
 __all__ = ["MultifidelityDataFusion", "AbstractMFGP", "NARGP", "GPDF", "GPDFC", "AbstractMaximizer",
-           "CandidateSetMaximizer", "LBFGSBMaximizer", "ScipyDirectMaximizer", "AbstractAugmIterator",
+           "ALCMaximizer", "CandidateSetMaximizer", "LBFGSBMaximizer", "ScipyDirectMaximizer", "AbstractAugmIterator",
            "BackwardAugmentation", "EvenAugmentation"]

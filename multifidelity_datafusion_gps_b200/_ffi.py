@@ -27,6 +27,7 @@ EXPORTS = [
     "mfgp_predict_mc_delays", "mfgp_fill_normal",
     "mfgp_predictive_gradients_ws_bytes", "mfgp_predictive_gradients",
     "mfgp_argmax", "mfgp_acq_batch_ws_bytes", "mfgp_acq_batch_begin", "mfgp_acq_batch_step",
+    "mfgp_alc_ws_bytes", "mfgp_alc",
     "mfgp_pce_ws_bytes", "mfgp_pce_project",
 ]
 
@@ -116,6 +117,9 @@ def load_library():
     lib.mfgp_predictive_gradients_ws_bytes.argtypes = [c_int, c_ll]
     lib.mfgp_predictive_gradients_ws_bytes.restype = c_sz
     lib.mfgp_predictive_gradients.argtypes = [vp, ctypes.POINTER(Level), vp, c_ll, vp, vp, vp, vp, c_int, vp, c_sz]
+    lib.mfgp_alc_ws_bytes.argtypes = [c_int, c_ll, c_ll]
+    lib.mfgp_alc_ws_bytes.restype = c_sz
+    lib.mfgp_alc.argtypes = [vp, ctypes.POINTER(Level), vp, c_ll, vp, c_ll, vp, c_dbl, vp, vp, c_sz]
     lib.mfgp_acq_batch_ws_bytes.argtypes = [c_int, c_ll, c_int]
     lib.mfgp_acq_batch_ws_bytes.restype = c_sz
     lib.mfgp_acq_batch_begin.argtypes = [vp, ctypes.POINTER(Level), vp, c_ll, c_int, c_int, vp, c_sz, vp, vp, vp]
@@ -128,7 +132,7 @@ def load_library():
         fn = getattr(lib, name)
         if name not in ("mfgp_last_error", "mfgp_launch_count", "mfgp_predict_ws_bytes", "mfgp_pce_ws_bytes",
                         "mfgp_predict_mc_joint_ws_bytes", "mfgp_predict_mc_ws_bytes", "mfgp_point_service_relaunches",
-                        "mfgp_acq_batch_ws_bytes", "mfgp_predictive_gradients_ws_bytes"):
+                        "mfgp_acq_batch_ws_bytes", "mfgp_predictive_gradients_ws_bytes", "mfgp_alc_ws_bytes"):
             fn.restype = c_int
     _lib = lib
     return lib

@@ -689,6 +689,116 @@ constexpr size_t xgrad_smem(int D) {
   return fm::EXP_TBL_BYTES + ((size_t)D * BT + 2 * ((size_t)D * GK + GK + (size_t)BT * GU_LD)) * sizeof(double);
 }
 
+// ---- K8c: integrated-variance (ALC) reduction ------------------------------------------------------------------
+//   alc[c] = sum_r w_r (k(c, r) - G[c][r])^2 / (kdiag - sum_i Tt[c][i]^2 + s2),  -inf where the denominator is <= 0
+// with G = Tt_C Tt_R^T (the latent posterior covariance is k - G).  The layout is cross_grad_kernel's: a CTA owns
+// 128 candidates and walks the reference rows in double-buffered stages of GK (cp.async: their rows, weights, and
+// the matching 128 x GK block of G).  Thread t serves candidate t/2 and the stage's references r = 2m + t%2; the two
+// partial sums meet in one shuffle, and the squared norm of the Tt row is summed the same way, so every value runs
+// in a fixed order that depends on nothing but R and npad.  w == nullptr: every weight is w_def.
+template <int DT, int E>
+__global__ void __launch_bounds__(256, 2)
+    alc_reduce_kernel(KParams kp, const double* __restrict__ Xr, long R, const double* __restrict__ w, double w_def,
+                      const double* __restrict__ G, long ldg, const double* __restrict__ Tt, int npad,
+                      const double* __restrict__ Xc, long ncols, double s2, double* __restrict__ alc) {
+  extern __shared__ __align__(16) double dsm[];   // exp table | sXc[D][BT] | 2 x (sXr[D][GK] | w[GK] | sG[BT][GU_LD])
+  const int D = DT > 0 ? DT : kp.D, d = DT > 0 ? DT - E : kp.d;
+  double* sXc = dsm + fm::EXP_TBL_DOUBLES;
+  double* sSt = sXc + D * BT;
+  const int stage = D * GK + GK + BT * GU_LD;
+  fm::load_exp_table(dsm, kp.exp_tbl);
+  const KEval<DT, E> ke(kp, fm::lane_table(dsm));
+  const long c0 = (long)blockIdx.x * BT;
+  const int cl = threadIdx.x >> 1, h = threadIdx.x & 1;
+  {
+    const long left = ncols - c0;
+    prefetch_rows<DT>(sXc, Xc + c0 * D, left > BT ? BT : (int)left, D, 0);
+  }
+  auto prefetch = [&](long s, int buf) {
+    double* p = sSt + buf * stage;
+    const long r0 = s * GK;
+    for (int i = threadIdx.x; i < GK * D; i += blockDim.x) {   // rows r0.. are one contiguous run of Xr
+      const int r = i / D, dd = i - r * D;
+      const bool ok = r0 + r < R;
+      cp_async8_zfill(p + dd * GK + r, ok ? Xr + r0 * D + i : Xr, ok);
+    }
+    if (threadIdx.x < GK) {
+      const bool ok = r0 + (long)threadIdx.x < R;
+      if (w) cp_async8_zfill(p + D * GK + threadIdx.x, ok ? w + r0 + threadIdx.x : w, ok);
+      else p[D * GK + threadIdx.x] = ok ? w_def : 0.0;
+    }
+    double* sg = p + D * GK + GK;
+    for (int i = threadIdx.x; i < BT * GK; i += blockDim.x) {
+      const int r = i / GK, kk = i - r * GK;
+      const bool ok = c0 + r < ncols && r0 + kk < R;
+      cp_async8_zfill(sg + r * GU_LD + kk, ok ? G + (c0 + r) * ldg + r0 + kk : G, ok);
+    }
+  };
+  const long nst = (R + GK - 1) / GK;
+  prefetch(0, 0);
+  cp_async_commit();
+  // |W k_c|^2 from the candidate's Tt row while the first stage lands: thread h takes the pairs 4m + 2h, 4m + 2h + 1
+  double sq = 0.0;
+  {
+    const long c = c0 + cl < ncols ? c0 + cl : c0;
+    const double2* row = reinterpret_cast<const double2*>(Tt + c * (long)npad);
+    for (int m = 0; m < npad / 4; m++) {
+      const double2 t = row[2 * m + h];
+      sq = fma(t.x, t.x, sq);
+      sq = fma(t.y, t.y, sq);
+    }
+  }
+  double q[DT > 0 ? DT : 1];
+  double acc = 0.0;
+  int buf = 0;
+  for (long s = 0; s < nst; s++, buf ^= 1) {
+    if (s + 1 < nst) prefetch(s + 1, buf ^ 1);
+    cp_async_commit();
+    cp_async_wait<1>();
+    __syncthreads();
+    if (DT > 0 && s == 0) {
+#pragma unroll
+      for (int dd = 0; dd < (DT > 0 ? DT : 1); dd++) q[dd] = sXc[dd * BT + cl];
+    }
+    const double* sXr = sSt + buf * stage;
+    const double* sW = sXr + D * GK;
+    const double* sG = sW + GK;
+#pragma unroll 2
+    for (int m = 0; m < GK / 2; m++) {
+      const int k = 2 * m + h;
+      double rx = 0.0, rz = 0.0;
+      if (DT > 0) {
+#pragma unroll
+        for (int dd = 0; dd < (DT > 0 ? DT : 1); dd++) {
+          const double t = q[dd] - sXr[dd * GK + k];
+          if (dd < DT - E) rx = fma(t, t, rx);
+          else rz = fma(t, t, rz);
+        }
+      } else {
+        for (int dd = 0; dd < D; dd++) {
+          const double t = sXc[dd * BT + cl] - sXr[dd * GK + k];
+          if (dd < d) rx = fma(t, t, rx);
+          else rz = fma(t, t, rz);
+        }
+      }
+      double kv = ke.k12(rx, rz);
+      if (ke.has3) kv += ke.k3(rx);
+      const double g = kv - sG[cl * GU_LD + k];
+      acc = fma(sW[k] * g, g, acc);
+    }
+    __syncthreads();   // all readers done with this buffer before the next iteration refills it
+  }
+  cp_async_wait<0>();
+  acc += __shfl_xor_sync(0xffffffffu, acc, 1);
+  sq += __shfl_xor_sync(0xffffffffu, sq, 1);
+  const long c = c0 + cl;
+  if (h != 0 || c >= ncols) return;
+  const double den = (kp.kdiag - sq) + s2;
+  alc[c] = den > 0.0 ? acc / den : -INFINITY;
+}
+
+constexpr size_t alc_smem(int D) { return xgrad_smem(D); }
+
 constexpr size_t asm_smem(int D) { return fm::EXP_TBL_BYTES + (size_t)2 * 2 * D * BT * sizeof(double); }
 constexpr size_t grad_smem(int D) { return fm::EXP_TBL_BYTES + (size_t)2 * 2 * (D + 1) * BT * sizeof(double); }
 
@@ -706,6 +816,8 @@ int assemble_configure(mfgp_ctx* h) {
   CUDA_TRY(h, cudaFuncSetAttribute(grad_reduce_kernel<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, gmax));
   CUDA_TRY(h, cudaFuncSetAttribute(cross_grad_kernel<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                    (int)xgrad_smem(MFGP_MAX_D)));
+  CUDA_TRY(h, cudaFuncSetAttribute(alc_reduce_kernel<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                   (int)alc_smem(MFGP_MAX_D)));
 #define MFGP_CFG(DT, E)                                                                                   \
   CUDA_TRY(h, cudaFuncSetAttribute(assemble_kernel<true, DT, E>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
                                    (int)asm_smem(DT)));                                                   \
@@ -714,7 +826,9 @@ int assemble_configure(mfgp_ctx* h) {
   CUDA_TRY(h, cudaFuncSetAttribute(cross_tile_kernel<DT, E>, cudaFuncAttributeMaxDynamicSharedMemorySize,     \
                                    (int)cross_smem(DT)));                                                 \
   CUDA_TRY(h, cudaFuncSetAttribute(cross_grad_kernel<DT, E>, cudaFuncAttributeMaxDynamicSharedMemorySize,     \
-                                   (int)xgrad_smem(DT)));
+                                   (int)xgrad_smem(DT)));                                                 \
+  CUDA_TRY(h, cudaFuncSetAttribute(alc_reduce_kernel<DT, E>, cudaFuncAttributeMaxDynamicSharedMemorySize,     \
+                                   (int)alc_smem(DT)));
   MFGP_SHAPES(MFGP_CFG)
 #undef MFGP_CFG
   return 0;
@@ -827,6 +941,32 @@ int cross_grad_launch(mfgp_ctx* h, const KParams& kp, const double* X, int N, co
       cross_grad_kernel<0, 0><<<grid, 256, smem, h->stream>>>(kp, X, N, alpha, Ut, (long)ldu, Xq, (long)ncols, j0,
                                                               dmean, dvar, mean, quad);
   prof_end(h, PC_CROSSGEN);
+  LAUNCH_CHECK(h);
+  return 0;
+}
+
+// K8c launcher: alc of the candidates Xc[0, ncols) (see alc_reduce_kernel), timed as acquisition work (class 9).
+int alc_reduce_launch(mfgp_ctx* h, const KParams& kp, const double* Xr, long long R, const double* w, double w_def,
+                      const double* G, long long ldg, const double* Tt, int npad, const double* Xc, long long ncols,
+                      double s2, double* alc) {
+  if (ncols <= 0) return 0;
+  const Shape sh = shape_of(kp);
+  const unsigned grid = (unsigned)((ncols + BT - 1) / BT);
+  const size_t smem = alc_smem(kp.D);
+  prof_begin(h, PC_ARGMAX);
+  bool done = false;
+#define MFGP_RUN(DT_, E_)                                                                                      \
+  if (!done && sh.DT == DT_ && sh.E == E_) {                                                                   \
+    alc_reduce_kernel<DT_, E_><<<grid, 256, smem, h->stream>>>(kp, Xr, (long)R, w, w_def, G, (long)ldg, Tt, npad, \
+                                                               Xc, (long)ncols, s2, alc);                      \
+    done = true;                                                                                               \
+  }
+  MFGP_SHAPES(MFGP_RUN)
+#undef MFGP_RUN
+  if (!done)
+    alc_reduce_kernel<0, 0><<<grid, 256, smem, h->stream>>>(kp, Xr, (long)R, w, w_def, G, (long)ldg, Tt, npad, Xc,
+                                                            (long)ncols, s2, alc);
+  prof_end(h, PC_ARGMAX);
   LAUNCH_CHECK(h);
   return 0;
 }

@@ -1284,4 +1284,59 @@ int mfgp_acq_batch_step(mfgp_handle_t h, const mfgp_level_t* gp, const double* d
   return acq_finish(h, L, d_cands, D, C, i + 1, q, h_val, h_idx, h_rec);
 }
 
+// ---- K8c integrated-variance (ALC) acquisition (math: assemble.cu, alc_reduce_kernel) ---------------------------
+// Scratch: Ks_R | Tt_R (Rpad x npad each) | per chunk Ks, Tt_C (chunk x npad each) | G (chunk x Rpad).
+constexpr long long ALC_MAX_R = (1LL << 31) - 128;   // Rpad is a GEMM extent (int)
+
+static long long alc_fixed_doubles(int N, long long R) {
+  return 2LL * ((R + 127) / 128 * 128) * mfgp_padded_n(N);
+}
+static long long alc_col_doubles(int N, long long R) { return 2LL * mfgp_padded_n(N) + (R + 127) / 128 * 128; }
+
+size_t mfgp_alc_ws_bytes(int N, long long C, long long R) {
+  if (N < 1 || C < 1 || R < 1 || R > ALC_MAX_R) return 0;
+  const unsigned long long cap = 1ULL << 30, per_col = 8ULL * alc_col_doubles(N, R);
+  const unsigned long long cpad = (unsigned long long)((C + 127) / 128 * 128);
+  unsigned long long chunk = cpad > cap / per_col ? cap : per_col * cpad;   // what C columns need, capped
+  if (chunk < 128 * per_col) chunk = 128 * per_col;                          // at least one 128-column chunk
+  return (size_t)(8ULL * alc_fixed_doubles(N, R) + chunk);
+}
+
+int mfgp_alc(mfgp_handle_t h, const mfgp_level_t* gp, const double* d_cands, long long C, const double* d_ref,
+             long long R, const double* d_w, double jitter, double* d_alc, double* d_ws, size_t ws_bytes) {
+  ENTER(h);
+  KParams kp;
+  int rc = level_kparams(h, gp, &kp);
+  if (rc) return rc;
+  ARG_CHECK(h, gp->d_W != nullptr && d_cands && d_ref && d_alc && d_ws);
+  ARG_CHECK(h, C >= 1 && R >= 1 && R <= ALC_MAX_R && std::isfinite(jitter) && jitter >= 0.0);
+  const int N = gp->N, npad = mfgp_padded_n(N);
+  const long long rpad = (R + 127) / 128 * 128, fixed = alc_fixed_doubles(N, R), per_col = alc_col_doubles(N, R);
+  const long long have = (long long)(ws_bytes / sizeof(double));
+  ARG_CHECK(h, have >= fixed + 128 * per_col);
+  long long chunk = whole_waves((have - fixed) / per_col / 128 * 128);
+  const long long max_chunk = whole_waves(1LL << 30);   // keeps the chunk a GEMM extent (int) whatever ws_bytes is
+  if (chunk > max_chunk) chunk = max_chunk;
+  double* KsR = d_ws;
+  double* TtR = KsR + rpad * npad;
+  double* Ks = TtR + rpad * npad;
+  double* TtC = Ks + chunk * npad;
+  double* G = TtC + chunk * npad;
+  const double s2 = kp.noise + JITTER_CONST + jitter;
+  if ((rc = cross_gen_launch(h, kp, gp->d_X, N, npad, gp->d_alpha, d_ref, R, rpad, KsR, nullptr))) return rc;
+  if ((rc = trmm_rows(h, gp->d_W, npad, KsR, rpad, TtR))) return rc;
+  for (long long c0 = 0; c0 < C; c0 += chunk) {
+    const long long ncols = (C - c0 < chunk) ? (C - c0) : chunk;
+    const long long cols_pad = (ncols + 127) / 128 * 128;
+    const double* Xc = d_cands + c0 * gp->D;
+    if ((rc = cross_gen_launch(h, kp, gp->d_X, N, npad, gp->d_alpha, Xc, ncols, cols_pad, Ks, nullptr))) return rc;
+    if ((rc = trmm_rows(h, gp->d_W, npad, Ks, cols_pad, TtC))) return rc;
+    if ((rc = gemm_nt(h, TtC, npad, TtR, npad, G, rpad, cols_pad, rpad, npad))) return rc;
+    if ((rc = alc_reduce_launch(h, kp, d_ref, R, d_w, 1.0 / (double)R, G, rpad, TtC, npad, Xc, ncols, s2,
+                                d_alc + c0)))
+      return rc;
+  }
+  return 0;
+}
+
 }  // extern "C"

@@ -170,6 +170,11 @@ int small_batch_max();
 int small_lml_batch_launch(mfgp_ctx* h, const KParams* kps, const double* diag_add, int B, const double* X,
                            const double* y, int N, double* d_out, int* d_info, int want_grad);
 int trmm_store(mfgp_ctx* h, const double* W, int npad, const double* Ks, long long cols_pad, double* T);
+// Tt = Ks W^T for the rows of Ks (cols_pad x npad, like Tt): the first product of kinv_rows
+int trmm_rows(mfgp_ctx* h, const double* W, int npad, const double* Ks, long long cols_pad, double* Tt);
+// C (m x n, ld ldc) = A B^T for A (m x k, ld lda) and B (n x k, ld ldb); m, n multiples of 128, k of LEAF
+int gemm_nt(mfgp_ctx* h, const double* A, long long lda, const double* B, long long ldb, double* C, long long ldc,
+            long long m, long long n, int k);
 // Ut = Ks K_y^-1 for the rows of Ks (cols_pad x npad, like Ut and the scratch Tt), Wt = W^T (npad x npad)
 int kinv_rows(mfgp_ctx* h, const double* W, const double* Wt, int npad, const double* Ks, long long cols_pad,
               double* Tt, double* Ut);
@@ -189,5 +194,8 @@ int cross_tile_launch(mfgp_ctx* h, const KParams& kp, const double* X, int N, in
 int cross_grad_launch(mfgp_ctx* h, const KParams& kp, const double* X, int N, const double* alpha, const double* Ut,
                       long long ldu, const double* Xq, long long ncols, double* dmean, double* dvar, double* mean,
                       double* quad);
+int alc_reduce_launch(mfgp_ctx* h, const KParams& kp, const double* Xr, long long R, const double* w, double w_def,
+                      const double* G, long long ldg, const double* Tt, int npad, const double* Xc, long long ncols,
+                      double s2, double* alc);
 int grad_reduce_launch(mfgp_ctx* h, const KParams& kp, const double* X, int N, const double* Kinv,
                        long long ld, const double* alpha, double* d_out8);

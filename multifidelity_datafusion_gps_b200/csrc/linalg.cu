@@ -1082,17 +1082,31 @@ int trmm_store(mfgp_ctx* h, const double* W, int npad, const double* Ks, long lo
 // one accumulation order, so a row's result does not depend on how many rows share the call.  (U = W^T T as a TT
 // product would go through gemm_tma_mc_kernel from one wave of tiles on, whose k order differs.)
 //   Tt[c][i] = sum_{k<=i} Ks[c][k] W[i][k],   Ut[c][k] = sum_{i>=k} Tt[c][i] Wt[k][i]
-int kinv_rows(mfgp_ctx* h, const double* W, const double* Wt, int npad, const double* Ks, long long cols_pad,
-              double* Tt, double* Ut) {
+int trmm_rows(mfgp_ctx* h, const double* W, int npad, const double* Ks, long long cols_pad, double* Tt) {
   ARG_CHECK(h, npad % LEAF == 0 && cols_pad % dg::Big16::BM == 0 && cols_pad < (1LL << 31));
   if (cols_pad == 0) return 0;
   dg::GemmParams p = gp(Ks, npad, W, npad, Tt, npad, (int)cols_pad, npad, npad, 1.0, 0.0);
   p.ke_col = 1;
-  int rc = launch_gemm<true, true>(h, p, PC_MISC);
-  if (rc) return rc;
-  p = gp(Tt, npad, Wt, npad, Ut, npad, (int)cols_pad, npad, npad, 1.0, 0.0);
+  return launch_gemm<true, true>(h, p, PC_MISC);
+}
+
+int kinv_rows(mfgp_ctx* h, const double* W, const double* Wt, int npad, const double* Ks, long long cols_pad,
+              double* Tt, double* Ut) {
+  int rc = trmm_rows(h, W, npad, Ks, cols_pad, Tt);
+  if (rc || cols_pad == 0) return rc;
+  dg::GemmParams p = gp(Tt, npad, Wt, npad, Ut, npad, (int)cols_pad, npad, npad, 1.0, 0.0);
   p.kb_col = 1;
   return launch_gemm<true, true>(h, p, PC_MISC);
+}
+
+// C[r][c] = sum_k A[r][k] B[c][k]: a plain NT product, so an entry depends only on its two operand rows
+int gemm_nt(mfgp_ctx* h, const double* A, long long lda, const double* B, long long ldb, double* C, long long ldc,
+            long long m, long long n, int k) {
+  ARG_CHECK(h, m % dg::Big16::BM == 0 && n % dg::Big16::BN == 0 && k % LEAF == 0);
+  ARG_CHECK(h, m < (1LL << 31) && n < (1LL << 31));
+  if (m == 0 || n == 0) return 0;
+  return launch_gemm<true, true>(h, gp(A, (long)lda, B, (long)ldb, C, (long)ldc, (int)m, (int)n, k, 1.0, 0.0),
+                                 PC_GEMM);
 }
 
 __global__ void transpose_kernel(const double* __restrict__ A, int n, double* __restrict__ At) {

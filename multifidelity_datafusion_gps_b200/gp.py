@@ -618,6 +618,36 @@ class GPRegression:
                                    ws_ptr, nbytes))
         return mean, var
 
+    def alc_device(self, dXc, dXr, dw=None, ws_bytes=None):
+        """Integrated-variance (ALC) acquisition values of the candidate rows dXc (C, D) over the reference rows dXr
+        (R, D), CUDA tensors -> (C,) CUDA tensor (mfgp_alc): alc[c] = sum_r w_r k_n(c, r)^2 / (v_n(c) + s^2), the drop
+        in the w-weighted latent variance at the references that append_point(c) at the current theta would cause;
+        -inf where v_n(c) + s^2 <= 0.  dw: (R,) CUDA weights, or None for 1/R.  ws_bytes: the scratch handed to the
+        call (default mfgp_alc_ws_bytes(N, C, R)); a candidate's value does not depend on it."""
+        h = _ffi.get_handle(self.device)
+        C, R = int(dXc.shape[0]), int(dXr.shape[0])
+        if dXc.ndim != 2 or dXr.ndim != 2 or int(dXc.shape[1]) != self.D or int(dXr.shape[1]) != self.D:
+            raise ValueError("candidate and reference rows must have the level's input width D = %d" % self.D)
+        if R < 1:
+            raise ValueError("the reference set is empty")
+        if dw is not None and tuple(dw.shape) != (R,):
+            raise ValueError("weights must have one entry per reference row (%d), got shape %s"
+                             % (R, tuple(dw.shape)))
+        lvl = self.level_struct()                           # settles last_jitter
+        dXc, dXr = dXc.contiguous(), dXr.contiguous()
+        dw = dw.contiguous() if dw is not None else None
+        assert dXc.dtype == dXr.dtype == torch.float64 and (dw is None or dw.dtype == torch.float64)
+        alc = torch.empty(C, dtype=torch.float64, device=dXc.device)
+        if C == 0:
+            return alc
+        if ws_bytes is None:
+            ws_bytes = h.lib.mfgp_alc_ws_bytes(self.N, C, R)
+        ws = workspace(self.device, ws_bytes)
+        h.check(h.lib.mfgp_alc(h.h, ctypes.byref(lvl), dXc.data_ptr(), C, dXr.data_ptr(), R,
+                               dw.data_ptr() if dw is not None else None, float(self.last_jitter),
+                               alc.data_ptr(), ws.data_ptr(), int(ws_bytes)))
+        return alc
+
     def predictive_gradients_device(self, dX, want_var=True, include_noise=True):
         """dX (M, D) CUDA -> (dmean (M, D), dvar (M, D) or None, mean (M,), var (M,) or None) CUDA tensors
         (mfgp_predictive_gradients).  dvar: gradient of the unclipped latent variance; mean and var: predict_device's
